@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU; torchrun for N > 1)
   python bench.py --impl reference --gpus N ...            the reference's own CPU implementation on the host cores
+  python bench.py ... --dump-outputs DIR                   also write the last timed step's outputs as DIR/<name>.npy
 
 A step = one pass of the hot path over one batch: F frames (default 100 000, BASELINE configs[1]) of the
 n=18432/m=2048 code, codeword[f % 272] through a BSC(eps), prprp max 100 iterations, decoded bits + iteration counts out.
@@ -21,6 +22,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; the bench writes nothing into it
+DUMP_FRAMES = 512              # --dump-outputs: frames whose decoded bits are written (18432 x 4 B each)
+DUMP_SCALAR_FRAMES = 1 << 20   # --dump-outputs: frames whose iteration count and codeword flag are written (8 B each)
 PCHK = os.path.join(ROOT, "tests", "golden", "decode_n18432_m2048_final.pchk")
 CW_BITS = os.path.join(ROOT, "tests", "golden", "codewords_n18432_272.bits")
 N, M, E = 18432, 2048, 147456
@@ -148,6 +152,31 @@ def _ev_time(torch, fn, reps=1):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / reps
+
+
+def _sample_frames(F, k):
+    """All F frame indices, or k of them drawn with a fixed seed (sorted): the same frames on every run."""
+    return np.arange(F) if F <= k else np.sort(np.random.default_rng(0).choice(F, k, replace=False))
+
+
+def dump_outputs(out_dir, d_bits, d_it, d_ok):
+    """What the caller of dnaldpc_decode_batch_device receives, as float .npy files: iteration counts and codeword flags
+    (frames.npy: which frames, all of them up to DUMP_SCALAR_FRAMES) and the decoded bits, unpacked to 0/1, of
+    DUMP_FRAMES frames (bits_frames.npy). Under 64 MB in all; the inputs depend on the arguments alone, so two builds run
+    with the same arguments can be compared file by file."""
+    import torch
+    F = d_it.shape[0]
+    os.makedirs(out_dir, exist_ok=True)
+    idx = _sample_frames(F, DUMP_SCALAR_FRAMES)
+    sel = torch.from_numpy(idx).to(d_it.device)
+    np.save(os.path.join(out_dir, "frames.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "iters.npy"), d_it[sel].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "is_codeword.npy"), d_ok[sel].cpu().numpy().astype(np.float32))
+    idx = _sample_frames(F, DUMP_FRAMES)
+    words = d_bits[torch.from_numpy(idx).to(d_bits.device)].cpu().numpy()
+    bits = np.unpackbits(words.view(np.uint8), axis=1, bitorder="little")[:, :N]
+    np.save(os.path.join(out_dir, "bits_frames.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "bits.npy"), bits.astype(np.float32))
 
 
 def secondary_regimes(ldpc, torch, dec, code, d_cw, args, peak):
@@ -444,6 +473,8 @@ def run_ours(args):
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
     frame_iters = int(d_it.sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_bits, d_it, d_ok)
     ms, frame_iters_all = aggregate(ms, frame_iters, dev, world)
     value = world * F * args.steps * N / (ms * 1e-3) / 1e9
 
@@ -602,7 +633,7 @@ def main():
     ap.add_argument("--max-iter", type=int, default=100)
     ap.add_argument("--wave", type=int, default=4096)
     ap.add_argument("--seed", type=int, default=7)
-    ap.add_argument("--e2e-steps", type=int, default=3)
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the host-buffer leg (default: --steps)")
     ap.add_argument("--ref-frames-per-core", type=int, default=4)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary regimes (converging frames, configs 3-5, fp32, min-sum, host-buffer kinds)")
@@ -610,7 +641,13 @@ def main():
     ap.add_argument("--inproc-frames", type=int, default=1000000, help="N > 1: frames of the one batch rank 0 decodes through the library's own multi-GPU dispatch")
     ap.add_argument("--alg", default="bp", choices=["bp", "minsum"], help="bp = sum-product (the metric); minsum = floating min-sum (SURVEY 8f-4)")
     ap.add_argument("--precision", default="f64", choices=["f64", "f32"], help="f64 = bit-exact mode (the metric); f32 = optional fast mode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the decoded bits, iteration counts and codeword flags of the last timed step (rank 0) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

@@ -2,6 +2,7 @@
 tools/make_golden.py): same argv (the pipeline's call, ex_decoder/def_func.py:49), same files in, byte-identical
 stdout / dec_*.txt and identical result_*.txt apart from the two wall-clock lines."""
 import hashlib
+import json
 import os
 import shutil
 import subprocess
@@ -79,91 +80,108 @@ def test_cli_errors_and_batch_list(tmp_path):
     assert b"frame_num              : 5" in r.stdout and b"bit_err                : 0" in r.stdout
 
 
+# The side-by-side cases below compare our CLI with the unmodified reference CLI (oracle/_ref/ldpc_ref). What the
+# reference printed and wrote for each case is kept in tests/golden/cli_side_by_side.json (tools/make_golden_cli_side.py),
+# so the comparison runs without the reference build; where it is built, the live reference CLI is compared as well.
 REF_CLI = os.path.join(ROOT, "oracle", "_ref", "ldpc_ref")
+GOLDEN_SIDE = os.path.join(ol.GOLDEN, "cli_side_by_side.json")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="oracle/_ref/ldpc_ref not built")
-@pytest.mark.parametrize("dectype", ["0", "20"])
-def test_cli_side_by_side_with_reference_binary(tmp_path, dectype):
-    """Our CLI and the unmodified reference CLI (prebuilt oracle/_ref/ldpc_ref) on the same files: BP (type 0) and
-    floating min-sum (type 20, Run_MSA_Decoder_INF)."""
+def _record(r, d, dec_name, keep=lambda line: True):
+    """stdout, SHA-256 of the dec file, result-file name and its body without the wall-clock lines: JSON-able."""
+    assert r.returncode == 0, r.stderr
+    res = [f for f in os.listdir(d) if f.startswith("result_")]
+    assert len(res) == 1
+    return {"stdout": r.stdout.decode("latin-1"),
+            "dec_sha256": hashlib.sha256(open(os.path.join(d, dec_name), "rb").read()).hexdigest(),
+            "result_name": res[0], "result": [line for line in _strip_times(open(os.path.join(d, res[0])).read()) if keep(line)]}
+
+
+def _bp_case(exe, d, dectype):
     cws = ol.load_codewords()
+    shutil.copyfile(ol.PCHK_18432, os.path.join(d, "H.pchk"))
+    eps = 0.005
+    llr = np.where((cws[3] ^ ol.bsc_flips(17, 3, 18432, eps)) == 0, 1.0, -1.0) * np.log((1 - eps) / eps) * np.linspace(0.7, 1.3, 18432)
+    cwname, softname = _write_inputs(d, 3, llr, cws)
+    r = subprocess.run([exe, "0", dectype, "0", "7", "60", "1", cwname, softname, "H", "0", "0", "0", "0"], cwd=d, capture_output=True)
+    return _record(r, d, "dec_%s.txt" % cwname)
+
+
+def _sw_case(exe, d, _=None):
+    g = np.load(os.path.join(ol.GOLDEN, "golden_sw.npz"))
+    N = 768
+    rs = np.random.RandomState(8)
+    llr = np.where(rs.rand(N) < 0.05, -1.0, 1.0) * rs.uniform(1.0, 4.0, N)
+    shutil.copyfile(os.path.join(ol.GOLDEN, "sc_z32_l12.pchk"), os.path.join(d, "sc.pchk"))
+    with open(os.path.join(d, "sc.txt"), "w") as fh:
+        fh.write("".join("%d\n" % v for v in g["Mv"]) + "".join("%d\n" % v for v in g["Mc"]))
+    with open(os.path.join(d, "cw.txt"), "w") as fh:
+        fh.write("0 " * N)
+    with open(os.path.join(d, "soft.txt"), "w") as fh:
+        fh.write(" ".join(repr(float(x)) for x in llr))
+    r = subprocess.run([exe, "0", "60", "0", "7", "20", "1", "cw", "soft", "sc", "0", "0", "0", "0", "0", "3", "12", "4"], cwd=d, capture_output=True)
+    return _record(r, d, "dec_cw.txt", keep=lambda line: not line.startswith("BER["))
+
+
+def _args_case(exe, d, args):
+    N = 768
+    rs = np.random.RandomState(12)
+    llr = np.where(rs.rand(N) < 0.04, -1.0, 1.0) * rs.uniform(0.5, 4.0, N)
+    shutil.copyfile(os.path.join(ol.GOLDEN, "sc_z32_l12.pchk"), os.path.join(d, "sc.pchk"))
+    with open(os.path.join(d, "cw.txt"), "w") as fh:
+        fh.write("0 " * N)
+    with open(os.path.join(d, "soft.txt"), "w") as fh:
+        fh.write(" ".join(repr(float(x)) for x in llr))
+    r = subprocess.run([exe] + list(args), cwd=d, capture_output=True)
+    return _record(r, d, "dec_cw.txt")
+
+
+ARG_VARIANTS = [
+    ("1", "0", "1", "7", "20", "3", "cw", "soft", "sc", "0.05", "0", "0", "0"),    # systematic count, BSC naming (%.4f), frame_num 3
+    ("0", "0", "2", "5", "10", "1", "cw", "soft", "sc", "0.3", "0", "0", "0"),     # BEC naming / "Eps" lines
+    ("0", "21", "0", "9", "15", "2", "cw", "soft", "sc", "1.5", "0", "0", "0"),    # min-sum type 21, Eb/N0 1.5 dB -> g_std_dev
+    ("0", "0", "0", "7", "0", "1", "cw", "soft", "sc", "0", "0", "0", "0"),        # max_iter 0
+]
+# name -> (case, its parameter); the names key tests/golden/cli_side_by_side.json
+SIDE_CASES = dict([("bp type 0", (_bp_case, "0")), ("bp type 20", (_bp_case, "20")), ("sw type 60", (_sw_case, None))]
+                  + [("args " + " ".join(a), (_args_case, a)) for a in ARG_VARIANTS])
+
+
+def _side_by_side(tmp_path, name):
+    case, param = SIDE_CASES[name]
     outs = {}
     for who, exe in (("ours", LDPC), ("ref", REF_CLI)):
+        if who == "ref" and not os.path.exists(REF_CLI):
+            continue
         d = str(tmp_path / who)
         os.makedirs(d)
-        shutil.copyfile(ol.PCHK_18432, os.path.join(d, "H.pchk"))
-        eps = 0.005
-        llr = np.where((cws[3] ^ ol.bsc_flips(17, 3, 18432, eps)) == 0, 1.0, -1.0) * np.log((1 - eps) / eps) * np.linspace(0.7, 1.3, 18432)
-        cwname, softname = _write_inputs(d, 3, llr, cws)
-        r = subprocess.run([exe, "0", dectype, "0", "7", "60", "1", cwname, softname, "H", "0", "0", "0", "0"], cwd=d, capture_output=True)
-        assert r.returncode == 0, r.stderr
-        res = [f for f in os.listdir(d) if f.startswith("result_")]
-        assert len(res) == 1
-        outs[who] = (r.stdout, open(os.path.join(d, "dec_%s.txt" % cwname), "rb").read(), res[0],
-                     _strip_times(open(os.path.join(d, res[0])).read()))
-    assert outs["ours"] == outs["ref"]
+        outs[who] = case(exe, d, param)
+    assert outs["ours"] == json.load(open(GOLDEN_SIDE))["cases"][name]
+    if "ref" in outs:
+        assert outs["ours"] == outs["ref"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="oracle/_ref/ldpc_ref not built")
+@pytest.mark.parametrize("dectype", ["0", "20"])
+def test_cli_side_by_side_with_reference_binary(tmp_path, dectype):
+    """Our CLI and the unmodified reference CLI on the same files: BP (type 0) and floating min-sum (type 20,
+    Run_MSA_Decoder_INF)."""
+    _side_by_side(tmp_path, "bp type " + dectype)
+
+
 def test_cli_sliding_window_side_by_side(tmp_path):
     """Decoder type 60 (sliding-window BP, Run_SW_Decoder) with the reference's own argument block
     `<code_type> <w> <L> <WIN>` and node-count file <pchk_base>.txt: stdout, dec file, result-file name and the result
     file up to its BER lines (which the reference computes from an uninitialised counter, SURVEY section 5) must equal the
     unmodified reference CLI's. The POSITION_BER diagnostic file is not produced."""
-    g = np.load(os.path.join(ol.GOLDEN, "golden_sw.npz"))
-    N, D = 768, 14
-    rs = np.random.RandomState(8)
-    llr = np.where(rs.rand(N) < 0.05, -1.0, 1.0) * rs.uniform(1.0, 4.0, N)
-    outs = {}
-    for who, exe in (("ours", LDPC), ("ref", REF_CLI)):
-        d = str(tmp_path / who)
-        os.makedirs(d)
-        shutil.copyfile(os.path.join(ol.GOLDEN, "sc_z32_l12.pchk"), os.path.join(d, "sc.pchk"))
-        with open(os.path.join(d, "sc.txt"), "w") as fh:
-            fh.write("".join("%d\n" % v for v in g["Mv"]) + "".join("%d\n" % v for v in g["Mc"]))
-        with open(os.path.join(d, "cw.txt"), "w") as fh:
-            fh.write("0 " * N)
-        with open(os.path.join(d, "soft.txt"), "w") as fh:
-            fh.write(" ".join(repr(float(x)) for x in llr))
-        r = subprocess.run([exe, "0", "60", "0", "7", "20", "1", "cw", "soft", "sc", "0", "0", "0", "0", "0", "3", "12", "4"], cwd=d, capture_output=True)
-        assert r.returncode == 0, r.stderr
-        res = [f for f in os.listdir(d) if f.startswith("result_")]
-        assert len(res) == 1
-        body = _strip_times(open(os.path.join(d, res[0])).read())
-        outs[who] = (r.stdout, open(os.path.join(d, "dec_cw.txt"), "rb").read(), res[0], [l for l in body if not l.startswith("BER[")])
-    assert outs["ours"] == outs["ref"]
-    assert len(g["Mv"]) == D
+    _side_by_side(tmp_path, "sw type 60")
+    assert len(np.load(os.path.join(ol.GOLDEN, "golden_sw.npz"))["Mv"]) == 14
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="oracle/_ref/ldpc_ref not built")
-@pytest.mark.parametrize("args", [
-    ("1", "0", "1", "7", "20", "3", "cw", "soft", "sc", "0.05", "0", "0", "0"),    # systematic count, BSC naming (%.4f), frame_num 3
-    ("0", "0", "2", "5", "10", "1", "cw", "soft", "sc", "0.3", "0", "0", "0"),     # BEC naming / "Eps" lines
-    ("0", "21", "0", "9", "15", "2", "cw", "soft", "sc", "1.5", "0", "0", "0"),    # min-sum type 21, Eb/N0 1.5 dB -> g_std_dev
-    ("0", "0", "0", "7", "0", "1", "cw", "soft", "sc", "0", "0", "0", "0"),        # max_iter 0
-])
+@pytest.mark.parametrize("args", ARG_VARIANTS)
 def test_cli_argument_variants_side_by_side(tmp_path, args):
     """The positional arguments the pipeline never varies (bSystematic, channel type + parameter, frame_num, seed,
     max_iter 0) against the unmodified reference CLI on the small SC code: stdout, dec file, result-file name and body."""
-    N = 768
-    rs = np.random.RandomState(12)
-    llr = np.where(rs.rand(N) < 0.04, -1.0, 1.0) * rs.uniform(0.5, 4.0, N)
-    outs = {}
-    for who, exe in (("ours", LDPC), ("ref", REF_CLI)):
-        d = str(tmp_path / who)
-        os.makedirs(d)
-        shutil.copyfile(os.path.join(ol.GOLDEN, "sc_z32_l12.pchk"), os.path.join(d, "sc.pchk"))
-        with open(os.path.join(d, "cw.txt"), "w") as fh:
-            fh.write("0 " * N)
-        with open(os.path.join(d, "soft.txt"), "w") as fh:
-            fh.write(" ".join(repr(float(x)) for x in llr))
-        r = subprocess.run([exe] + list(args), cwd=d, capture_output=True)
-        assert r.returncode == 0, r.stderr
-        res = [f for f in os.listdir(d) if f.startswith("result_")]
-        assert len(res) == 1
-        outs[who] = (r.stdout, open(os.path.join(d, "dec_cw.txt"), "rb").read(), res[0], _strip_times(open(os.path.join(d, res[0])).read()))
-    assert outs["ours"] == outs["ref"]
+    _side_by_side(tmp_path, "args " + " ".join(args))
 
 
 def test_resident_worker_serves_the_unmodified_command_line(tmp_path):
