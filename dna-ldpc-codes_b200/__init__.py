@@ -26,7 +26,8 @@ EXPORTS = [
     "dnaldpc_decode_batch_device", "dnaldpc_run_bp_decoder", "dnaldpc_std_dev", "dnaldpc_vote_table",
     "dnaldpc_bsc_table", "dnaldpc_synth_bsc_device", "dnaldpc_get_stats", "dnaldpc_set_profiling",
     "dnaldpc_selftest_math", "dnaldpc_redecode_sweep", "dnaldpc_get_trace", "dnaldpc_decode_window",
-    "dnaldpc_redecode_sweep_ex", "dnaldpc_synth_awgn_device", "dnaldpc_synth_vote_device",
+    "dnaldpc_redecode_sweep_ex", "dnaldpc_synth_awgn_device", "dnaldpc_synth_vote_device", "dnaldpc_code_systematic",
+    "dnaldpc_encode_device", "dnaldpc_encode", "dnaldpc_extract_device", "dnaldpc_extract",
 ]
 
 
@@ -108,6 +109,11 @@ def lib():
         L.dnaldpc_synth_vote_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_int64, C.c_int64,
                                                 C.c_double, C.c_double, C.c_void_p, C.c_void_p]
         L.dnaldpc_decode_window.argtypes = [C.c_void_p, C.POINTER(Window), C.c_void_p, C.c_int64, C.c_int, C.POINTER(Output)]
+        L.dnaldpc_code_systematic.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.c_void_p]
+        for name in ("dnaldpc_encode_device", "dnaldpc_extract_device"):
+            getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+        for name in ("dnaldpc_encode", "dnaldpc_extract"):
+            getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
         _lib = L
     return _lib
 
@@ -152,6 +158,30 @@ class Code:
 
     def write_pchk(self, path):
         _check(lib().dnaldpc_code_write_pchk(self._h, os.fsencode(path)))
+
+    def systematic(self):
+        """(info_cols, parity_cols) of the systematic form (include/dnaldpc.h): K = len(info_cols) = N - rank(H)."""
+        if getattr(self, "_sys", None) is None:
+            K = C.c_int()
+            info = np.zeros(self.N, np.int32); par = np.zeros(self.N, np.int32)
+            _check(lib().dnaldpc_code_systematic(self._h, C.byref(K), info.ctypes.data, par.ctypes.data))
+            self._sys = (info[:K.value].copy(), par[:self.N - K.value].copy())
+        return self._sys
+
+
+def _pack_bits(bits):
+    """int8 / bool [F][n] -> uint32 [F][ceil(n/32)], LSB first."""
+    bits = np.asarray(bits)
+    F, n = bits.shape
+    w = (n + 31) // 32
+    b = np.zeros((F, w * 32), np.uint8)
+    b[:, :n] = bits != 0
+    return np.ascontiguousarray(np.packbits(b, axis=1, bitorder="little")).view(np.uint32)
+
+
+def _unpack_bits(words, n):
+    F = words.shape[0]
+    return np.unpackbits(words.view(np.uint8).reshape(F, -1), axis=1, bitorder="little")[:, :n].astype(np.int8)
 
 
 _KIND_DTYPE = {IN_LR_F64: np.float64, IN_LLR_F64: np.float64, IN_BSC_BITS: np.uint32, IN_AWGN_F32: np.float32,
@@ -295,6 +325,38 @@ class Decoder:
         inp = Input(kind=kind, flags=flags, data=data_ptr, frame_stride=frame_stride, param=param, table=table_ptr)
         out = Output(bits=bits_ptr, dblk=dblk_ptr, iters=iters_ptr, is_codeword=ok_ptr, posterior=post_ptr, pchk=pchk_ptr)
         _check(lib().dnaldpc_decode_batch_device(self._h, C.byref(inp), F, max_iter, C.byref(out), stream))
+
+    @property
+    def K(self):
+        return len(self.code.systematic()[0])
+
+    def encode(self, msg):
+        """HOST numpy: message bits int8 [F][K] -> codewords int8 [F][N] (systematic form of include/dnaldpc.h)."""
+        msg = np.asarray(msg)
+        assert msg.ndim == 2 and msg.shape[1] == self.K, msg.shape
+        F = msg.shape[0]
+        m = _pack_bits(msg)
+        cw = np.zeros((F, self.words_per_frame), np.uint32)
+        _check(lib().dnaldpc_encode(self._h, m.ctypes.data, F, cw.ctypes.data))
+        return _unpack_bits(cw, self.code.N)
+
+    def extract(self, bits):
+        """HOST numpy: codeword bits int8 [F][N] -> message bits int8 [F][K] (the bits at the info columns)."""
+        bits = np.asarray(bits)
+        assert bits.ndim == 2 and bits.shape[1] == self.code.N, bits.shape
+        F, K = bits.shape[0], self.K
+        c = _pack_bits(bits)
+        m = np.zeros((F, (K + 31) // 32), np.uint32)
+        _check(lib().dnaldpc_extract(self._h, c.ctypes.data, F, m.ctypes.data))
+        return _unpack_bits(m, K)
+
+    def encode_device(self, msg_ptr, F, cw_ptr, stream=None):
+        """DEVICE pointers (ints) on the decoder's first GPU: uint32 [F][ceil(K/32)] -> uint32 [F][ceil(N/32)]."""
+        _check(lib().dnaldpc_encode_device(self._h, msg_ptr, F, cw_ptr, stream))
+
+    def extract_device(self, cw_ptr, F, msg_ptr, stream=None):
+        """DEVICE pointers (ints): uint32 [F][ceil(N/32)] -> uint32 [F][ceil(K/32)]."""
+        _check(lib().dnaldpc_extract_device(self._h, cw_ptr, F, msg_ptr, stream))
 
     def synth_bsc_device(self, cw_bits_ptr, n_cw, seed, frame0, F, eps, out_bits_ptr, stream=None):
         _check(lib().dnaldpc_synth_bsc_device(self._h, cw_bits_ptr, n_cw, seed, frame0, F, eps, out_bits_ptr, stream))

@@ -10,6 +10,8 @@
 
 #include "../../include/dnaldpc.h"
 #include "../host/code.h"
+#include "../host/systematic.h"
+#include "encoder.h"
 #include "engine.h"
 #include "sources.h"
 
@@ -22,6 +24,7 @@ struct dnaldpc_decoder {
     Code c;
     std::vector<std::unique_ptr<Engine>> eng;
     dnaldpc_stats stats{};
+    std::unique_ptr<Encoder> enc;  // on eng[0]'s device, created by the first encode / extract call
 };
 
 // Every entry point leaves the calling thread's current CUDA device as it found it (the engines switch devices).
@@ -381,6 +384,74 @@ int dnaldpc_synth_vote_device(dnaldpc_decoder *d, const uint32_t *cw_bits, int n
     if (!d) return set_err(DNALDPC_ERR_ARG, "null decoder");
     int rc = d->eng[0]->synth_vote(cw_bits, n_cw, seed, frame0, F, mean_reads, read_err, out_k, (cudaStream_t)stream);
     return rc ? set_err(rc, d->eng[0]->error()) : DNALDPC_OK;
+}
+
+int dnaldpc_code_systematic(const dnaldpc_code *c, int *K, int32_t *info_cols, int32_t *parity_cols) {
+    if (!c || !K) return set_err(DNALDPC_ERR_ARG, "null argument");
+    int rc = 0;
+    std::string err;
+    const Systematic *s = systematic_form(c->c, &rc, &err);
+    if (!s) return set_err(rc, err);
+    *K = s->K;
+    if (info_cols) memcpy(info_cols, s->info_cols.data(), s->info_cols.size() * 4);
+    if (parity_cols) memcpy(parity_cols, s->parity_cols.data(), s->parity_cols.size() * 4);
+    return DNALDPC_OK;
+}
+
+// Argument checks shared by the encode / extract entry points; *enc receives the decoder's encoder (created on first use).
+static int encoder_call(dnaldpc_decoder *d, const void *src, int64_t F, const void *dst, Encoder **enc) {
+    *enc = nullptr;
+    if (!d) return set_err(DNALDPC_ERR_ARG, "null decoder");
+    if (F < 0) return set_err(DNALDPC_ERR_ARG, "negative frame count");
+    if (F == 0) return DNALDPC_OK;
+    if (!src || !dst) return set_err(DNALDPC_ERR_ARG, "null buffer");
+    if (!d->enc) {
+        int rc = 0;
+        std::string err;
+        const Systematic *s = systematic_form(d->c, &rc, &err);
+        if (!s) return set_err(rc, err);
+        std::unique_ptr<Encoder> e(new Encoder(*s, d->c.N, d->eng[0]->device()));
+        if (!e->ok()) return set_err(DNALDPC_ERR_CUDA, e->error());
+        d->enc = std::move(e);
+    }
+    *enc = d->enc.get();
+    return DNALDPC_OK;
+}
+
+int dnaldpc_encode_device(dnaldpc_decoder *d, const uint32_t *msg, int64_t F, uint32_t *cw, void *stream) {
+    DeviceRestore restore_device;
+    Encoder *e;
+    int rc = encoder_call(d, msg, F, cw, &e);
+    if (rc || !e) return rc;
+    rc = e->encode(msg, F, cw, (cudaStream_t)stream);
+    return rc ? set_err(rc, e->error()) : DNALDPC_OK;
+}
+
+int dnaldpc_encode(dnaldpc_decoder *d, const uint32_t *msg, int64_t F, uint32_t *cw) {
+    DeviceRestore restore_device;
+    Encoder *e;
+    int rc = encoder_call(d, msg, F, cw, &e);
+    if (rc || !e) return rc;
+    rc = e->encode_host(msg, F, cw);
+    return rc ? set_err(rc, e->error()) : DNALDPC_OK;
+}
+
+int dnaldpc_extract_device(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg, void *stream) {
+    DeviceRestore restore_device;
+    Encoder *e;
+    int rc = encoder_call(d, cw, F, msg, &e);
+    if (rc || !e) return rc;
+    rc = e->extract(cw, F, msg, (cudaStream_t)stream);
+    return rc ? set_err(rc, e->error()) : DNALDPC_OK;
+}
+
+int dnaldpc_extract(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg) {
+    DeviceRestore restore_device;
+    Encoder *e;
+    int rc = encoder_call(d, cw, F, msg, &e);
+    if (rc || !e) return rc;
+    rc = e->extract_host(cw, F, msg);
+    return rc ? set_err(rc, e->error()) : DNALDPC_OK;
 }
 
 int dnaldpc_get_stats(const dnaldpc_decoder *d, dnaldpc_stats *s) {

@@ -3,10 +3,13 @@
 #include <algorithm>
 #include <cstdio>
 
+#include "systematic.h"
+
 namespace dnaldpc {
 
 std::string build_code(int M, int N, std::vector<int64_t> &pairs, Code &c) {
     if (M <= 0 || N <= 0) return "matrix dimensions must be positive";
+    c.sys = std::make_shared<SystematicCache>();
     std::sort(pairs.begin(), pairs.end());
     pairs.erase(std::unique(pairs.begin(), pairs.end()), pairs.end());  // insert() merges duplicates (mod2sparse.cpp:521-524)
     c.M = M; c.N = N; c.E = (int)pairs.size();

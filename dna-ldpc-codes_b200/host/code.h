@@ -4,10 +4,13 @@
 // ascending row; mod2sparse_insert, mod2sparse.cpp:502-604), which fix the floating-point product order.
 #pragma once
 #include <cstdint>
+#include <memory>
 #include <string>
 #include <vector>
 
 namespace dnaldpc {
+
+struct SystematicCache;
 
 struct Code {
     int M = 0, N = 0, E = 0;
@@ -17,6 +20,7 @@ struct Code {
     std::vector<int32_t> col_edge;  // [E]   CSR edge ids of column j, ascending row
     int max_row_deg = 0, max_col_deg = 0;
     bool regular_rows = true, regular_cols = true;
+    std::shared_ptr<SystematicCache> sys;  // systematic form (host/systematic.h), computed on first use
 };
 
 // Build from (row, col) pairs in any order with duplicates; returns error text or "".

@@ -27,6 +27,13 @@
 //                     same stdout, same exit code); otherwise it runs locally. The unmodified pipeline
 //                     (ex_decoder/def_func.py:47-51, one os.system("ldpc ...") per codeword) then pays milliseconds
 //                     per call instead of a CUDA context creation.
+//
+// Encoder (no counterpart in the reference's command line):
+//   ldpc --encode <pchk_base> <msg_base> <codeword_base>   or   ldpc --encode <pchk_base> --list FILE
+// reads K = N - rank(H) message bits (whitespace-separated 0/1) from <msg_base>.txt, encodes them on the GPU with the
+// systematic form of include/dnaldpc.h and writes <codeword_base>.txt in the codeword-file format (N x "%d ", no
+// newline) that the decode command line reads. --list FILE holds one "<msg_base> <codeword_base>" pair per line, all
+// encoded in one call. --device N and --timing apply; argument and file errors are reported before any CUDA call.
 #include <sys/socket.h>
 #include <sys/stat.h>
 #include <sys/un.h>
@@ -63,8 +70,9 @@ struct Args {
     int punctuation = 0, shortening = 0, targeting = 0;
     int sc_code_type = 0, sc_w = 0, sc_L = 0, sc_win = 0;  // decoder type 60 only
     int device = 0, gpus = 1;
-    bool fp32 = false, timing = false, serve = false, shutdown = false;
+    bool fp32 = false, timing = false, serve = false, shutdown = false, encode = false;
     std::string list, socket_path;
+    std::string msg_base;  // --encode: <pchk_base> <msg_base> <codeword_base> (cw_base, pchk_base as for decoding)
 };
 
 // Where a run writes: a local run uses the process's own streams, a run on behalf of a client memory streams.
@@ -85,9 +93,19 @@ bool parse(const std::vector<std::string> &argv, Args &a, Io &io) {
         else if (s == "--shutdown") a.shutdown = true;
         else if (s == "--socket" && i + 1 < argv.size()) a.socket_path = argv[++i];
         else if (s == "--list" && i + 1 < argv.size()) a.list = argv[++i];
+        else if (s == "--encode") a.encode = true;
         else pos.push_back(s);
     }
     if (a.serve || a.shutdown) return true;
+    if (a.encode) {
+        if (pos.size() != (a.list.empty() ? 3u : 1u)) {
+            fprintf(io.err, "usage: ldpc --encode <pchk_base> <msg_base> <codeword_base>  |  ldpc --encode <pchk_base> --list FILE\n");
+            return false;
+        }
+        a.pchk_base = pos[0];
+        if (a.list.empty()) { a.msg_base = pos[1]; a.cw_base = pos[2]; }
+        return true;
+    }
     size_t p = 0;
     bool short_of = false;
     auto next = [&]() -> const char * { if (p >= pos.size()) { short_of = true; return "0"; } return pos[p++].c_str(); };
@@ -406,6 +424,69 @@ int run(Args a, Io &io, Cache *cache) {
 #undef CHECK
 }
 
+// ldpc --encode: message files -> codeword files. Everything that can fail on the host (the parity-check file, the
+// systematic form, the message files) is checked before the GPU is touched.
+int run_encode(Args a, Io &io, bool resident) {
+    const std::string pchk_file = a.pchk_base + ".pchk";
+    dnaldpc_code *code = nullptr;
+    dnaldpc_decoder *dec = nullptr;
+    struct Owned {
+        dnaldpc_code *&code; dnaldpc_decoder *&dec;
+        ~Owned() { if (dec) dnaldpc_decoder_destroy(dec); if (code) dnaldpc_code_free(code); }
+    } owned{code, dec};
+    if (dnaldpc_code_read_pchk(io.path(pchk_file).c_str(), &code) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    int M, N, E, K;
+    dnaldpc_code_dims(code, &M, &N, &E);
+    if (dnaldpc_code_systematic(code, &K, nullptr, nullptr) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    std::vector<std::pair<std::string, std::string>> frames;  // (msg_base, codeword_base)
+    if (a.list.empty()) frames.push_back({a.msg_base, a.cw_base});
+    else {
+        FILE *f = fopen(io.path(a.list).c_str(), "r");
+        if (!f) { fprintf(io.err, "Can't open list file: %s\n", a.list.c_str()); return 1; }
+        char c1[512], c2[512];
+        while (fscanf(f, "%511s %511s", c1, c2) == 2) frames.push_back({c1, c2});
+        fclose(f);
+        if (frames.empty()) { fprintf(io.err, "List file %s holds no \"<msg> <codeword>\" pairs\n", a.list.c_str()); return 1; }
+    }
+    const size_t F = frames.size(), kw = (size_t)(K + 31) / 32, wpf = (size_t)(N + 31) / 32;
+    std::vector<uint32_t> msg(F * kw, 0u), cw(F * wpf, 0u);
+    std::string err;
+    for (size_t f = 0; f < F; f++) {
+        std::vector<signed char> m;
+        const std::string path = frames[f].first + ".txt";
+        if (!read_codeword_txt(io.path(path), K, m, err)) { fprintf(io.err, "%s\n", err.c_str()); return 1; }
+        for (int t = 0; t < K; t++) {
+            if (m[(size_t)t] != 0 && m[(size_t)t] != 1) { fprintf(io.err, "File %s holds a value other than 0 or 1\n", path.c_str()); return 1; }
+            msg[f * kw + (size_t)t / 32] |= (uint32_t)m[(size_t)t] << (t % 32);
+        }
+    }
+    if (a.device < 0) { fprintf(io.err, "ldpc: --device must be >= 0\n"); return 1; }
+    if (!resident && getenv("CUDA_VISIBLE_DEVICES") == nullptr) {  // as for decoding: initialise only the requested GPU
+        char dev[16];
+        snprintf(dev, sizeof(dev), "%d", a.device);
+        if (setenv("CUDA_VISIBLE_DEVICES", dev, 0) == 0) a.device = 0;
+    }
+    dnaldpc_config cfg{};
+    cfg.n_devices = 1;
+    cfg.devices[0] = a.device;
+    cfg.wave_frames = 32;
+    auto i0 = std::chrono::steady_clock::now();
+    if (dnaldpc_decoder_create(code, &cfg, &dec) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    auto c0 = std::chrono::steady_clock::now();
+    if (dnaldpc_encode(dec, msg.data(), (int64_t)F, cw.data()) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    auto c1 = std::chrono::steady_clock::now();
+    std::vector<unsigned char> bits((size_t)N);
+    for (size_t f = 0; f < F; f++) {
+        for (int j = 0; j < N; j++) bits[(size_t)j] = (unsigned char)((cw[f * wpf + (size_t)j / 32] >> (j % 32)) & 1u);
+        if (!write_dec_txt(io.path(frames[f].second + ".txt"), bits.data(), N, err)) { fprintf(io.err, "%s\n", err.c_str()); return 1; }
+    }
+    fprintf(io.out, "encoded %zu frame(s): N = %d, K = %d, M = %d\n", F, N, K, M);
+    if (a.timing)
+        fprintf(io.err, "{\"frames\": %zu, \"gpu_init_ms\": %.1f, \"encode_ms\": %.3f}\n", F,
+                std::chrono::duration<double, std::milli>(c0 - i0).count(), std::chrono::duration<double, std::milli>(c1 - c0).count());
+    return 0;
+}
+
 // ---- resident worker and its client ----------------------------------------------------------------------------
 // Wire format (host byte order, one request per connection): u32 magic, u32 argc, argc x (u32 length, bytes), u32 length +
 // bytes of the client's working directory; answer: i32 exit code, u32 length + bytes of stdout, u32 length + bytes of stderr.
@@ -505,7 +586,7 @@ int serve(const std::string &sock) {
             else if (parse(args, a, io)) {
                 if (a.shutdown) { stop = true; code = 0; }
                 else if (a.serve) { fprintf(io.err, "ldpc: a worker is already serving on this socket\n"); }
-                else code = run(a, io, &cache);
+                else code = a.encode ? run_encode(a, io, true) : run(a, io, &cache);
             }
             fclose(io.out);
             fclose(io.err);
@@ -536,5 +617,5 @@ int main(int argc, char **argv) {
         if (run_remote(sock, args, &rc)) return rc;
         if (a.shutdown) { fprintf(stderr, "ldpc: no worker answers on %s\n", sock.c_str()); return 1; }
     } else if (a.shutdown) { fprintf(stderr, "ldpc --shutdown: set DNALDPC_SOCKET or pass --socket PATH\n"); return 1; }
-    return run(a, io, nullptr);
+    return a.encode ? run_encode(a, io, false) : run(a, io, nullptr);
 }

@@ -195,6 +195,27 @@ int dnaldpc_synth_awgn_device(dnaldpc_decoder *d, const uint32_t *cw_bits, int n
 int dnaldpc_synth_vote_device(dnaldpc_decoder *d, const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0,
                               int64_t F, double mean_reads, double read_err, int8_t *out_k, void *stream);
 
+/* ---- systematic encoder ------------------------------------------------------------------------ */
+/* Systematic form of H. Scanning the columns from N-1 down to 0, column j is a parity column iff it is linearly
+ * independent over GF(2) of the parity columns already chosen (the pivot columns of the reduced row-echelon form of H
+ * with its column order reversed); a column with no entries is always an info column. R = rank(H) parity columns,
+ * K = N - R info columns, both lists ascending. Message bit t goes to info_cols[t]; parity bit i, at parity_cols[i], is
+ * XOR_t A[i][t] m_t, where row i of A is the reduced row whose pivot is parity_cols[i], restricted to the info columns.
+ * Hence encode(c[info_cols]) == c for every codeword c. Computed once per code, on first use (about a second for
+ * N = 18432); DNALDPC_ERR_UNSUPPORTED when M*M or R*K exceeds 2^33 bits.
+ * K receives N - rank(H); info_cols / parity_cols (capacity N each, may be NULL) receive the ascending column lists.
+ * Host only, no GPU needed. */
+int dnaldpc_code_systematic(const dnaldpc_code *c, int *K, int32_t *info_cols, int32_t *parity_cols);
+/* msg: uint32 [F][ceil(K/32)] LSB first (bits beyond K in the last word are ignored) -> cw: uint32 [F][ceil(N/32)] (the
+ * layout of dnaldpc_output.bits and of the synth functions' cw_bits; bits beyond N are written as 0). DEVICE buffers on
+ * the decoder's first device, asynchronous on `stream`. Encoding runs on that one device only (no multi-GPU dispatch). */
+int dnaldpc_encode_device(dnaldpc_decoder *d, const uint32_t *msg, int64_t F, uint32_t *cw, void *stream);
+int dnaldpc_encode(dnaldpc_decoder *d, const uint32_t *msg, int64_t F, uint32_t *cw);        /* HOST buffers, blocking */
+/* cw: uint32 [F][ceil(N/32)] -> msg: uint32 [F][ceil(K/32)], the bits at info_cols (no syndrome check; bits beyond K are
+ * written as 0). */
+int dnaldpc_extract_device(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg, void *stream);
+int dnaldpc_extract(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg);       /* HOST buffers, blocking */
+
 /* ---- statistics of the last decode call on this handle ------------------------------------------ */
 typedef struct dnaldpc_stats {
     int64_t frames;
