@@ -27,7 +27,7 @@ EXPORTS = [
     "dnaldpc_bsc_table", "dnaldpc_synth_bsc_device", "dnaldpc_get_stats", "dnaldpc_set_profiling",
     "dnaldpc_selftest_math", "dnaldpc_redecode_sweep", "dnaldpc_get_trace", "dnaldpc_decode_window",
     "dnaldpc_redecode_sweep_ex", "dnaldpc_synth_awgn_device", "dnaldpc_synth_vote_device", "dnaldpc_code_systematic",
-    "dnaldpc_encode_device", "dnaldpc_encode", "dnaldpc_extract_device", "dnaldpc_extract",
+    "dnaldpc_encode_device", "dnaldpc_encode", "dnaldpc_extract_device", "dnaldpc_extract", "dnaldpc_simulate",
 ]
 
 
@@ -55,6 +55,16 @@ class Stats(C.Structure):
 class Window(C.Structure):
     _fields_ = [("code_type", C.c_int32), ("L", C.c_int32), ("w", C.c_int32), ("win", C.c_int32),
                 ("Mv", C.c_void_p), ("Mc", C.c_void_p)]
+
+
+class Sim(C.Structure):
+    _fields_ = [("channel", C.c_int32), ("flags", C.c_int32), ("param", C.c_double), ("mean_reads", C.c_double),
+                ("seed", C.c_uint64), ("max_iter", C.c_int32), ("max_frames", C.c_int64), ("target_frame_errors", C.c_int64)]
+
+
+class SimResult(C.Structure):
+    _fields_ = [(k, C.c_int64) for k in ("frames", "iterations", "frame_errors", "bit_errors", "msg_frame_errors",
+                                         "msg_bit_errors", "detected", "undetected", "raw_frame_errors", "raw_bit_errors")]
 
 
 class LdpcError(RuntimeError):
@@ -114,6 +124,7 @@ def lib():
             getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
         for name in ("dnaldpc_encode", "dnaldpc_extract"):
             getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+        L.dnaldpc_simulate.argtypes = [C.c_void_p, C.POINTER(Sim), C.POINTER(SimResult)]
         _lib = L
     return _lib
 
@@ -366,6 +377,16 @@ class Decoder:
 
     def synth_vote_device(self, cw_bits_ptr, n_cw, seed, frame0, F, mean_reads, read_err, out_k_ptr, stream=None):
         _check(lib().dnaldpc_synth_vote_device(self._h, cw_bits_ptr, n_cw, seed, frame0, F, mean_reads, read_err, out_k_ptr, stream))
+
+    def simulate(self, channel, param, max_iter, max_frames, target_frame_errors=0, seed=0, flags=0, mean_reads=0.0):
+        """Monte-Carlo error rates (dnaldpc_simulate): random codewords of the systematic encoder through the synthetic
+        channel `channel` (IN_BSC_BITS p, IN_AWGN_F32 sigma, IN_VOTE_I8 read error probability + mean_reads), decoded
+        and counted on the GPU; stops after the first `target_frame_errors` frame errors (0 = exactly max_frames)."""
+        spec = Sim(channel=channel, flags=flags, param=param, mean_reads=mean_reads, seed=seed, max_iter=max_iter,
+                   max_frames=max_frames, target_frame_errors=target_frame_errors)
+        r = SimResult()
+        _check(lib().dnaldpc_simulate(self._h, C.byref(spec), C.byref(r)))
+        return {k: getattr(r, k) for k, _ in SimResult._fields_}
 
     def stats(self):
         s = Stats()

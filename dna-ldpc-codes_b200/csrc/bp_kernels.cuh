@@ -19,6 +19,7 @@
 #include <stdint.h>
 
 #include "bp_math.cuh"
+#include "rng.cuh"
 
 namespace dnaldpc {
 
@@ -1311,29 +1312,19 @@ __global__ void init_sched_kernel(SchedArrays s, int G, unsigned int *counters, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Synthetic BSC input generator (benchmarks): counter RNG keyed by (seed, GLOBAL frame, bit).
-// Must stay identical to oracle/bp_oracle.c:orc_rng_u64 and tests/oraclelib.py:rng_u64 (the specification).
+// Synthetic BSC input generator (benchmarks, csrc/sim.cu): counter RNG of rng.cuh keyed by (seed, GLOBAL frame, bit).
+// Frame f is noise on codeword row (f + cw_off) % n_cw of cw_bits (cw_off = 0 for the C-ABI synth functions; the
+// simulator points cw_bits at a piece of its codeword ring and picks cw_off so that frame f0 + i reads row i).
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ __forceinline__ uint64_t mix64(uint64_t z) {
-    z ^= z >> 30; z *= 0xBF58476D1CE4E5B9ULL;
-    z ^= z >> 27; z *= 0x94D049BB133111EBULL;
-    z ^= z >> 31;
-    return z;
-}
-__host__ __device__ __forceinline__ uint64_t rng_u64(uint64_t seed, uint64_t frame, uint64_t bit, uint64_t stream) {
-    uint64_t x = mix64(seed * 0x9E3779B97F4A7C15ULL + frame + 0x632BE59BD9B4E019ULL);
-    return mix64(x ^ (bit * 0xD6E8FEB86659FD93ULL + stream * 0xA0761D6478BD642FULL + 0x2545F4914F6CDD1DULL));
-}
-
 __global__ void __launch_bounds__(256)
-synth_bsc_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t seed, long long frame0, long long F, int N,
-                 int words_per_frame, uint64_t thr, uint32_t *__restrict__ out) {
+synth_bsc_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t cw_off, uint64_t seed, long long frame0, long long F,
+                 int N, int words_per_frame, uint64_t thr, uint32_t *__restrict__ out) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= F * words_per_frame) return;
     const long long fl = t / words_per_frame;
     const int w = (int)(t - fl * words_per_frame);
     const uint64_t f = (uint64_t)(frame0 + fl);
-    uint32_t word = cw_bits ? cw_bits[(size_t)(f % (uint64_t)n_cw) * words_per_frame + w] : 0u;
+    uint32_t word = cw_bits ? cw_bits[(size_t)((f + cw_off) % (uint64_t)n_cw) * words_per_frame + w] : 0u;
     const uint64_t fkey = mix64(seed * 0x9E3779B97F4A7C15ULL + f + 0x632BE59BD9B4E019ULL);
     for (int b = 0; b < 32; b++) {
         const int j = w * 32 + b;
@@ -1351,14 +1342,14 @@ synth_bsc_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t seed, 
 // Host twin: oracle/bp_oracle.c:orc_synth_awgn (libm; agrees to the last fp32 ulp except where the fp64 values
 // straddle a rounding boundary). Keyed by the GLOBAL frame index like synth_bsc_kernel.
 __global__ void __launch_bounds__(256)
-synth_awgn_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t seed, long long frame0, long long F, int N,
-                  int words_per_frame, double sigma, float *__restrict__ out) {
+synth_awgn_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t cw_off, uint64_t seed, long long frame0, long long F,
+                  int N, int words_per_frame, double sigma, float *__restrict__ out) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= F * N) return;
     const long long fl = t / N;
     const int j = (int)(t - fl * N);
     const uint64_t f = (uint64_t)(frame0 + fl);
-    const uint32_t bit = cw_bits ? (cw_bits[(size_t)(f % (uint64_t)n_cw) * words_per_frame + (j >> 5)] >> (j & 31)) & 1u : 0u;
+    const uint32_t bit = cw_bits ? (cw_bits[(size_t)((f + cw_off) % (uint64_t)n_cw) * words_per_frame + (j >> 5)] >> (j & 31)) & 1u : 0u;
     const double u1 = ((double)(rng_u64(seed, f, (uint64_t)j, 4) >> 11) + 1.0) * (1.0 / 9007199254740992.0);
     const double u2 = (double)(rng_u64(seed, f, (uint64_t)j, 5) >> 11) * (1.0 / 9007199254740992.0);
     const double n = sqrt(-2.0 * log(u1)) * cos(6.283185307179586476925286766559 * u2);
@@ -1372,14 +1363,14 @@ synth_awgn_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t seed,
 // twin (oracle/bp_oracle.c:orc_synth_vote) is exact.
 constexpr int kVoteMaxReads = 64;
 __global__ void __launch_bounds__(256)
-synth_vote_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t seed, long long frame0, long long F, int N,
-                  int words_per_frame, const uint64_t *__restrict__ thr, uint64_t thr_err, int8_t *__restrict__ out) {
+synth_vote_kernel(const uint32_t *__restrict__ cw_bits, int n_cw, uint64_t cw_off, uint64_t seed, long long frame0, long long F,
+                  int N, int words_per_frame, const uint64_t *__restrict__ thr, uint64_t thr_err, int8_t *__restrict__ out) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= F * N) return;
     const long long fl = t / N;
     const int j = (int)(t - fl * N);
     const uint64_t f = (uint64_t)(frame0 + fl);
-    const uint32_t bit = cw_bits ? (cw_bits[(size_t)(f % (uint64_t)n_cw) * words_per_frame + (j >> 5)] >> (j & 31)) & 1u : 0u;
+    const uint32_t bit = cw_bits ? (cw_bits[(size_t)((f + cw_off) % (uint64_t)n_cw) * words_per_frame + (j >> 5)] >> (j & 31)) & 1u : 0u;
     const uint64_t u = rng_u64(seed, f, (uint64_t)j, 2) >> 11;
     int c = 0;
     while (c < kVoteMaxReads - 1 && u >= __ldg(thr + c)) c++;

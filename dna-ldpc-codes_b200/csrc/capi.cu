@@ -13,6 +13,7 @@
 #include "../host/systematic.h"
 #include "encoder.h"
 #include "engine.h"
+#include "sim.h"
 #include "sources.h"
 
 using namespace dnaldpc;
@@ -25,6 +26,7 @@ struct dnaldpc_decoder {
     std::vector<std::unique_ptr<Engine>> eng;
     dnaldpc_stats stats{};
     std::unique_ptr<Encoder> enc;  // on eng[0]'s device, created by the first encode / extract call
+    std::vector<std::unique_ptr<Encoder>> sim_enc;  // on eng[1..]'s devices, created by the first multi-GPU simulation
 };
 
 // Every entry point leaves the calling thread's current CUDA device as it found it (the engines switch devices).
@@ -398,13 +400,8 @@ int dnaldpc_code_systematic(const dnaldpc_code *c, int *K, int32_t *info_cols, i
     return DNALDPC_OK;
 }
 
-// Argument checks shared by the encode / extract entry points; *enc receives the decoder's encoder (created on first use).
-static int encoder_call(dnaldpc_decoder *d, const void *src, int64_t F, const void *dst, Encoder **enc) {
-    *enc = nullptr;
-    if (!d) return set_err(DNALDPC_ERR_ARG, "null decoder");
-    if (F < 0) return set_err(DNALDPC_ERR_ARG, "negative frame count");
-    if (F == 0) return DNALDPC_OK;
-    if (!src || !dst) return set_err(DNALDPC_ERR_ARG, "null buffer");
+// The decoder's encoder on its first device, created on first use.
+static int first_encoder(dnaldpc_decoder *d) {
     if (!d->enc) {
         int rc = 0;
         std::string err;
@@ -414,6 +411,18 @@ static int encoder_call(dnaldpc_decoder *d, const void *src, int64_t F, const vo
         if (!e->ok()) return set_err(DNALDPC_ERR_CUDA, e->error());
         d->enc = std::move(e);
     }
+    return DNALDPC_OK;
+}
+
+// Argument checks shared by the encode / extract entry points; *enc receives the decoder's encoder.
+static int encoder_call(dnaldpc_decoder *d, const void *src, int64_t F, const void *dst, Encoder **enc) {
+    *enc = nullptr;
+    if (!d) return set_err(DNALDPC_ERR_ARG, "null decoder");
+    if (F < 0) return set_err(DNALDPC_ERR_ARG, "negative frame count");
+    if (F == 0) return DNALDPC_OK;
+    if (!src || !dst) return set_err(DNALDPC_ERR_ARG, "null buffer");
+    const int rc = first_encoder(d);
+    if (rc) return rc;
     *enc = d->enc.get();
     return DNALDPC_OK;
 }
@@ -452,6 +461,39 @@ int dnaldpc_extract(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t 
     if (rc || !e) return rc;
     rc = e->extract_host(cw, F, msg);
     return rc ? set_err(rc, e->error()) : DNALDPC_OK;
+}
+
+int dnaldpc_simulate(dnaldpc_decoder *d, const dnaldpc_sim *s, dnaldpc_sim_result *r) {
+    DeviceRestore restore_device;
+    if (!d || !s || !r) return set_err(DNALDPC_ERR_ARG, "null argument");
+    if (s->channel != DNALDPC_IN_BSC_BITS && s->channel != DNALDPC_IN_AWGN_F32 && s->channel != DNALDPC_IN_VOTE_I8)
+        return set_err(DNALDPC_ERR_ARG, "unknown simulation channel (BSC_BITS, AWGN_F32 or VOTE_I8)");
+    if (s->flags & ~(DNALDPC_FLAG_MINSUM | DNALDPC_FLAG_FIXED_ITERS)) return set_err(DNALDPC_ERR_ARG, "unknown simulation flag");
+    if ((s->channel == DNALDPC_IN_BSC_BITS || s->channel == DNALDPC_IN_VOTE_I8) && !(s->param > 0.0 && s->param < 1.0))
+        return set_err(DNALDPC_ERR_ARG, "error probability must be in (0,1)");
+    if (s->channel == DNALDPC_IN_AWGN_F32 && !(s->param > 0.0)) return set_err(DNALDPC_ERR_ARG, "AWGN sigma must be positive");
+    if (s->channel == DNALDPC_IN_VOTE_I8 && !(s->mean_reads > 0.0 && s->mean_reads <= 32.0))
+        return set_err(DNALDPC_ERR_ARG, "mean reads must be in (0, 32]");
+    if (s->max_iter < 0 || s->max_frames < 1 || s->target_frame_errors < 0)
+        return set_err(DNALDPC_ERR_ARG, "max_iter < 0, max_frames < 1 or target_frame_errors < 0");
+    int rc = 0;
+    std::string err;
+    const Systematic *sys = systematic_form(d->c, &rc, &err);
+    if (!sys) return set_err(rc, err);
+    // every device encodes its own frames: engine 0 with the decoder's encoder, the others with encoders of their own
+    rc = first_encoder(d);
+    if (rc) return rc;
+    std::vector<Encoder *> encs{d->enc.get()};
+    for (size_t k = 1; k < d->eng.size(); k++) {
+        if (d->sim_enc.size() < k) {
+            std::unique_ptr<Encoder> e(new Encoder(*sys, d->c.N, d->eng[k]->device()));
+            if (!e->ok()) return set_err(DNALDPC_ERR_CUDA, e->error());
+            d->sim_enc.push_back(std::move(e));
+        }
+        encs.push_back(d->sim_enc[k - 1].get());
+    }
+    rc = simulate_batch(d->eng, encs, *sys, *s, *r, d->stats, err);
+    return rc ? set_err(rc, err) : DNALDPC_OK;
 }
 
 int dnaldpc_get_stats(const dnaldpc_decoder *d, dnaldpc_stats *s) {

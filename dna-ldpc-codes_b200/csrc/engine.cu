@@ -975,7 +975,7 @@ int Engine::sw_lockstep(const dnaldpc_window &w, const std::vector<int> &sched, 
 }
 
 int Engine::synth_bsc(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double eps,
-                      uint32_t *out_bits, cudaStream_t stream) {
+                      uint32_t *out_bits, cudaStream_t stream, uint64_t cw_off) {
     err_.clear();
     if (F < 0 || !out_bits || (cw_bits && n_cw <= 0) || !(eps >= 0.0 && eps <= 1.0)) return fail("bad argument", DNALDPC_ERR_ARG);
     CK(cudaSetDevice(device_));
@@ -983,19 +983,19 @@ int Engine::synth_bsc(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t 
     const long long total = (long long)F * wpf;
     if (total == 0) return DNALDPC_OK;
     const uint64_t thr = (uint64_t)(eps * 9007199254740992.0);
-    synth_bsc_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, seed, frame0, F, N_, wpf, thr, out_bits);
+    synth_bsc_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, cw_off, seed, frame0, F, N_, wpf, thr, out_bits);
     CK(cudaGetLastError());
     return DNALDPC_OK;
 }
 
 int Engine::synth_awgn(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double sigma,
-                       float *out_y, cudaStream_t stream) {
+                       float *out_y, cudaStream_t stream, uint64_t cw_off) {
     err_.clear();
     if (F < 0 || !out_y || (cw_bits && n_cw <= 0) || !(sigma >= 0.0)) return fail("bad argument", DNALDPC_ERR_ARG);
     CK(cudaSetDevice(device_));
     const long long total = (long long)F * N_;
     if (total == 0) return DNALDPC_OK;
-    synth_awgn_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, seed, frame0, F, N_, (N_ + 31) / 32, sigma, out_y);
+    synth_awgn_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, cw_off, seed, frame0, F, N_, (N_ + 31) / 32, sigma, out_y);
     CK(cudaGetLastError());
     return DNALDPC_OK;
 }
@@ -1012,7 +1012,7 @@ void vote_thresholds(double mean, uint64_t *thr) {
 }
 
 int Engine::synth_vote(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double mean_reads,
-                       double read_err, int8_t *out_k, cudaStream_t stream) {
+                       double read_err, int8_t *out_k, cudaStream_t stream, uint64_t cw_off) {
     err_.clear();
     if (F < 0 || !out_k || (cw_bits && n_cw <= 0) || !(mean_reads > 0.0 && mean_reads <= 32.0) || !(read_err >= 0.0 && read_err <= 1.0))
         return fail("bad argument (mean reads in (0, 32], read error in [0, 1])", DNALDPC_ERR_ARG);
@@ -1024,7 +1024,7 @@ int Engine::synth_vote(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t
     if (!d_synth_thr_) CK(cudaMalloc((void **)&d_synth_thr_, sizeof(thr)));
     CK(cudaMemcpyAsync(d_synth_thr_, thr, sizeof(thr), cudaMemcpyHostToDevice, stream));  // pageable: staged before the call returns
     const uint64_t thr_err = (uint64_t)(read_err * 9007199254740992.0);
-    synth_vote_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, seed, frame0, F, N_, (N_ + 31) / 32, d_synth_thr_, thr_err, out_k);
+    synth_vote_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(cw_bits, n_cw, cw_off, seed, frame0, F, N_, (N_ + 31) / 32, d_synth_thr_, thr_err, out_k);
     CK(cudaGetLastError());
     return DNALDPC_OK;
 }

@@ -66,12 +66,14 @@ class Engine {
     // Sliding-window BP for spatially-coupled codes (Run_SW_Decoder, dec.cpp:2092-2196); HOST pointers; blocking.
     int decode_window_host(const Code &code, const dnaldpc_window &w, const double *lratio, int64_t F, int max_iter,
                            const dnaldpc_output &out);
+    // Synthetic channel outputs of frames [frame0, frame0+F) (include/dnaldpc.h); frame f is noise on codeword row
+    // (f + cw_off) % n_cw (the C ABI passes 0; the simulator points the generators at rows of its codeword ring).
     int synth_bsc(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double eps,
-                  uint32_t *out_bits, cudaStream_t stream);
+                  uint32_t *out_bits, cudaStream_t stream, uint64_t cw_off = 0);
     int synth_awgn(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double sigma,
-                   float *out_y, cudaStream_t stream);
+                   float *out_y, cudaStream_t stream, uint64_t cw_off = 0);
     int synth_vote(const uint32_t *cw_bits, int n_cw, uint64_t seed, int64_t frame0, int64_t F, double mean_reads,
-                   double read_err, int8_t *out_k, cudaStream_t stream);
+                   double read_err, int8_t *out_k, cudaStream_t stream, uint64_t cw_off = 0);
 
     dnaldpc_stats stats{};
     bool profiling = false;

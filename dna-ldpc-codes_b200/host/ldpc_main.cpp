@@ -28,6 +28,20 @@
 //                     (ex_decoder/def_func.py:47-51, one os.system("ldpc ...") per codeword) then pays milliseconds
 //                     per call instead of a CUDA context creation.
 //
+// Simulation (the reference's frame_num / target_frame_err mode: random codewords through a synthetic channel):
+//   ldpc --simulate <pchk_base> <channel_type> <p1[,p2,...]> <seed> <max_iter> <frame_num> [<target_frame_err> if frame_num==0]
+//        [--max-frames N] [--reads R] [--decoder 0|20] [--device N] [--gpus N] [--fp32] [--timing]
+// runs dnaldpc_simulate once per parameter: frames carry random messages (RNG stream 1 of DESIGN.md §9) encoded with
+// the systematic form, go through the channel and are decoded and counted on the GPU. Channel types: 0 = AWGN, the
+// parameters are Eb/N0 in dB and sigma = getStd_dev(Eb/N0, K/N) with K = N - rank(H), the true rate of the code;
+// 1 = BSC with crossover probability p; 3 = vote counts of aligned reads, p = read error probability (also the
+// decoder's eps), --reads R mean reads per bit (required, in (0, 32]). 2 (BEC) and anything else are rejected.
+// frame_num > 0 simulates exactly that many frames; frame_num 0 runs until <target_frame_err> frame errors, capped by
+// --max-frames (default 10^9). --decoder 20 decodes with floating min-sum. Per parameter a Print_One_Result block
+// (DNA_main.cpp:1170-1182) plus msg_bit_err, undetected (zero syndrome, wrong codeword) and avg_iter lines; --timing
+// adds one JSON line per parameter on stderr with every counter and the wall time. Argument and file errors are
+// reported before any CUDA call.
+//
 // Encoder (no counterpart in the reference's command line):
 //   ldpc --encode <pchk_base> <msg_base> <codeword_base>   or   ldpc --encode <pchk_base> --list FILE
 // reads K = N - rank(H) message bits (whitespace-separated 0/1) from <msg_base>.txt, encodes them on the GPU with the
@@ -70,9 +84,11 @@ struct Args {
     int punctuation = 0, shortening = 0, targeting = 0;
     int sc_code_type = 0, sc_w = 0, sc_L = 0, sc_win = 0;  // decoder type 60 only
     int device = 0, gpus = 1;
-    bool fp32 = false, timing = false, serve = false, shutdown = false, encode = false;
+    bool fp32 = false, timing = false, serve = false, shutdown = false, encode = false, simulate = false;
     std::string list, socket_path;
     std::string msg_base;  // --encode: <pchk_base> <msg_base> <codeword_base> (cw_base, pchk_base as for decoding)
+    std::vector<std::string> sim_pos;  // --simulate: the positional arguments after the flag
+    std::string max_frames, reads, decoder;  // --simulate options, checked by run_simulate
 };
 
 // Where a run writes: a local run uses the process's own streams, a run on behalf of a client memory streams.
@@ -94,9 +110,14 @@ bool parse(const std::vector<std::string> &argv, Args &a, Io &io) {
         else if (s == "--socket" && i + 1 < argv.size()) a.socket_path = argv[++i];
         else if (s == "--list" && i + 1 < argv.size()) a.list = argv[++i];
         else if (s == "--encode") a.encode = true;
+        else if (s == "--simulate") a.simulate = true;
+        else if (s == "--max-frames" && i + 1 < argv.size()) a.max_frames = argv[++i];
+        else if (s == "--reads" && i + 1 < argv.size()) a.reads = argv[++i];
+        else if (s == "--decoder" && i + 1 < argv.size()) a.decoder = argv[++i];
         else pos.push_back(s);
     }
     if (a.serve || a.shutdown) return true;
+    if (a.simulate) { a.sim_pos = pos; return true; }
     if (a.encode) {
         if (pos.size() != (a.list.empty() ? 3u : 1u)) {
             fprintf(io.err, "usage: ldpc --encode <pchk_base> <msg_base> <codeword_base>  |  ldpc --encode <pchk_base> --list FILE\n");
@@ -487,6 +508,133 @@ int run_encode(Args a, Io &io, bool resident) {
     return 0;
 }
 
+// ldpc --simulate: one dnaldpc_simulate call per channel parameter.
+const char kSimUsage[] =
+    "usage: ldpc --simulate <pchk_base> <channel_type> <p1[,p2,...]> <seed> <max_iter> <frame_num> [<target_frame_err> if frame_num==0]\n"
+    "                       [--max-frames N] [--reads R] [--decoder 0|20] [--device N] [--gpus N] [--fp32] [--timing]\n"
+    "  channel_type 0: AWGN, parameters Eb/N0 in dB, sigma from the true rate K/N (K = N - rank(H))\n"
+    "               1: BSC, parameters crossover probabilities p\n"
+    "               3: vote counts, parameters read error probabilities, --reads = mean reads per bit (required)\n";
+
+bool parse_num(const std::string &s, double &v) {
+    char *end = nullptr;
+    v = strtod(s.c_str(), &end);
+    return !s.empty() && end && *end == 0 && std::isfinite(v);
+}
+bool parse_int(const std::string &s, long long &v) {
+    char *end = nullptr;
+    v = strtoll(s.c_str(), &end, 10);
+    return !s.empty() && end && *end == 0;
+}
+
+int run_simulate(Args a, Io &io, bool resident) {
+    auto usage = [&](const char *why) {
+        if (why) fprintf(io.err, "ldpc --simulate: %s\n", why);
+        fputs(kSimUsage, io.err);
+        return 1;
+    };
+    const std::vector<std::string> &p = a.sim_pos;
+    if (p.size() < 6) return usage("too few arguments");
+    long long chan = 0, seed = 0, max_iter = 0, frame_num = 0, target = 0, max_frames = 1000000000LL;
+    if (!parse_int(p[1], chan)) return usage("channel_type is not an integer");
+    if (chan == 2) { fprintf(io.err, "ldpc --simulate: channel type 2 (BEC) is not supported by this build (0 = AWGN, 1 = BSC, 3 = vote counts)\n"); return 1; }
+    if (chan != 0 && chan != 1 && chan != 3) { fprintf(io.err, "ldpc --simulate: unknown channel type %lld (0 = AWGN, 1 = BSC, 3 = vote counts)\n", chan); return 1; }
+    if (!parse_int(p[3], seed) || seed < 0) return usage("seed must be a non-negative integer");
+    if (!parse_int(p[4], max_iter) || max_iter < 0 || max_iter > 0x7fffffff) return usage("max_iter must be a non-negative integer");
+    if (!parse_int(p[5], frame_num) || frame_num < 0) return usage("frame_num must be a non-negative integer");
+    if (frame_num == 0) {
+        if (p.size() != 7) return usage(p.size() < 7 ? "frame_num 0 needs <target_frame_err>" : "too many arguments");
+        if (!parse_int(p[6], target) || target < 1) return usage("target_frame_err must be a positive integer");
+        if (!a.max_frames.empty() && (!parse_int(a.max_frames, max_frames) || max_frames < 1)) return usage("--max-frames must be a positive integer");
+    } else if (p.size() != 6) return usage("too many arguments");
+    std::vector<double> params;
+    {
+        size_t b = 0;
+        for (;;) {
+            const size_t e = p[2].find(',', b);
+            double v = 0;
+            if (!parse_num(p[2].substr(b, e == std::string::npos ? std::string::npos : e - b), v)) return usage("bad channel parameter list");
+            if (chan != 0 && !(v > 0.0 && v < 1.0)) { fprintf(io.err, "ldpc --simulate: error probability %g is not in (0,1)\n", v); return 1; }
+            params.push_back(v);
+            if (e == std::string::npos) break;
+            b = e + 1;
+        }
+    }
+    double reads = 0;
+    if (chan == 3) {
+        if (a.reads.empty()) return usage("channel type 3 (vote counts) needs --reads R");
+        if (!parse_num(a.reads, reads) || !(reads > 0.0 && reads <= 32.0)) return usage("--reads must be in (0, 32]");
+    }
+    int flags = 0;
+    if (!a.decoder.empty() && a.decoder != "0") {
+        if (a.decoder != "20") return usage("--decoder must be 0 (belief propagation) or 20 (floating min-sum)");
+        flags = DNALDPC_FLAG_MINSUM;
+    }
+    if (a.device < 0) return usage("--device must be >= 0");
+    if (a.gpus < 1 || a.gpus > 16) return usage("--gpus must be between 1 and 16");
+
+    const std::string pchk_file = p[0] + ".pchk";
+    dnaldpc_code *code = nullptr;
+    dnaldpc_decoder *dec = nullptr;
+    struct Owned {
+        dnaldpc_code *&code; dnaldpc_decoder *&dec;
+        ~Owned() { if (dec) dnaldpc_decoder_destroy(dec); if (code) dnaldpc_code_free(code); }
+    } owned{code, dec};
+    if (dnaldpc_code_read_pchk(io.path(pchk_file).c_str(), &code) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    int M, N, E, K;
+    dnaldpc_code_dims(code, &M, &N, &E);
+    if (dnaldpc_code_systematic(code, &K, nullptr, nullptr) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    const double rate = (double)K / (double)N;
+
+    if (!resident && a.gpus == 1 && getenv("CUDA_VISIBLE_DEVICES") == nullptr) {  // as for decoding: initialise only the requested GPU
+        char dev[16];
+        snprintf(dev, sizeof(dev), "%d", a.device);
+        if (setenv("CUDA_VISIBLE_DEVICES", dev, 0) == 0) a.device = 0;
+    }
+    dnaldpc_config cfg{};
+    cfg.n_devices = a.gpus;
+    for (int k = 0; k < a.gpus; k++) cfg.devices[k] = a.device + k;
+    cfg.precision = a.fp32 ? DNALDPC_PREC_F32 : DNALDPC_PREC_F64;
+    if (dnaldpc_decoder_create(code, &cfg, &dec) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    fprintf(io.out, "\ng_CODE_N : %d\ng_CODE_K : %d\ng_CODE_M : %d\n\n", N, K, M);
+    for (size_t i = 0; i < params.size(); i++) {
+        dnaldpc_sim sp{};
+        sp.channel = chan == 0 ? DNALDPC_IN_AWGN_F32 : chan == 1 ? DNALDPC_IN_BSC_BITS : DNALDPC_IN_VOTE_I8;
+        sp.flags = flags;
+        sp.param = chan == 0 ? dnaldpc_std_dev(params[i], rate) : params[i];
+        sp.mean_reads = reads;
+        sp.seed = (uint64_t)seed;
+        sp.max_iter = (int32_t)max_iter;
+        sp.max_frames = frame_num > 0 ? frame_num : max_frames;
+        sp.target_frame_errors = frame_num > 0 ? 0 : target;
+        dnaldpc_sim_result r{};
+        const auto t0 = std::chrono::steady_clock::now();
+        if (dnaldpc_simulate(dec, &sp, &r) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+        const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        // Print_One_Result (DNA_main.cpp:1170-1182) and the counters the reference does not have
+        const int k = (int)i;
+        if (chan == 0) fprintf(io.out, "[%d]  code : (%d,%d)\trate : %.3f\tEb/No : %.2f dB\n", k, N, K, rate, params[i]);
+        else fprintf(io.out, "[%d]  code : (%d,%d)\trate : %.3f\tp : %.5f\n", k, N, K, rate, params[i]);
+        fprintf(io.out, "[%d]  frame_num              : %lld\n", k, (long long)r.frames);
+        fprintf(io.out, "[%d]  bit_err                : %lld\n", k, (long long)r.bit_errors);
+        fprintf(io.out, "[%d]  frame_err              : %lld\n", k, (long long)r.frame_errors);
+        fprintf(io.out, "[%d]  without coding (bit)   : %lld\n", k, (long long)r.raw_bit_errors);
+        fprintf(io.out, "[%d]  without coding (frame) : %lld\n", k, (long long)r.raw_frame_errors);
+        fprintf(io.out, "[%d]  msg_bit_err            : %lld\n", k, (long long)r.msg_bit_errors);
+        fprintf(io.out, "[%d]  undetected             : %lld\n", k, (long long)r.undetected);
+        fprintf(io.out, "[%d]  avg_iter               : %.4f\n\n", k, r.frames ? (double)r.iterations / (double)r.frames : 0.0);
+        fflush(io.out);
+        if (a.timing)
+            fprintf(io.err, "{\"point\": %d, \"channel_type\": %lld, \"param\": %.17g, \"channel_param\": %.17g, \"frames\": %lld, "
+                    "\"iterations\": %lld, \"frame_errors\": %lld, \"bit_errors\": %lld, \"msg_frame_errors\": %lld, \"msg_bit_errors\": %lld, "
+                    "\"detected\": %lld, \"undetected\": %lld, \"raw_frame_errors\": %lld, \"raw_bit_errors\": %lld, \"wall_ms\": %.3f}\n",
+                    k, chan, params[i], sp.param, (long long)r.frames, (long long)r.iterations, (long long)r.frame_errors,
+                    (long long)r.bit_errors, (long long)r.msg_frame_errors, (long long)r.msg_bit_errors, (long long)r.detected,
+                    (long long)r.undetected, (long long)r.raw_frame_errors, (long long)r.raw_bit_errors, ms);
+    }
+    return 0;
+}
+
 // ---- resident worker and its client ----------------------------------------------------------------------------
 // Wire format (host byte order, one request per connection): u32 magic, u32 argc, argc x (u32 length, bytes), u32 length +
 // bytes of the client's working directory; answer: i32 exit code, u32 length + bytes of stdout, u32 length + bytes of stderr.
@@ -586,7 +734,7 @@ int serve(const std::string &sock) {
             else if (parse(args, a, io)) {
                 if (a.shutdown) { stop = true; code = 0; }
                 else if (a.serve) { fprintf(io.err, "ldpc: a worker is already serving on this socket\n"); }
-                else code = a.encode ? run_encode(a, io, true) : run(a, io, &cache);
+                else code = a.encode ? run_encode(a, io, true) : a.simulate ? run_simulate(a, io, true) : run(a, io, &cache);
             }
             fclose(io.out);
             fclose(io.err);
@@ -617,5 +765,5 @@ int main(int argc, char **argv) {
         if (run_remote(sock, args, &rc)) return rc;
         if (a.shutdown) { fprintf(stderr, "ldpc: no worker answers on %s\n", sock.c_str()); return 1; }
     } else if (a.shutdown) { fprintf(stderr, "ldpc --shutdown: set DNALDPC_SOCKET or pass --socket PATH\n"); return 1; }
-    return a.encode ? run_encode(a, io, false) : run(a, io, nullptr);
+    return a.encode ? run_encode(a, io, false) : a.simulate ? run_simulate(a, io, false) : run(a, io, nullptr);
 }

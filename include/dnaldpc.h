@@ -216,6 +216,43 @@ int dnaldpc_encode(dnaldpc_decoder *d, const uint32_t *msg, int64_t F, uint32_t 
 int dnaldpc_extract_device(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg, void *stream);
 int dnaldpc_extract(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t *msg);       /* HOST buffers, blocking */
 
+/* ---- Monte-Carlo error-rate simulation ---------------------------------------------------------- */
+/* Random codewords through a synthetic channel, decoded and counted on the decoder's devices (Run_Simulation /
+ * Print_One_Result of the reference's command line). Contract:
+ *   Frames. Frame f (global index 0, 1, ...) carries the message whose 32-bit word w is the low 32 bits of
+ *     rng_u64(seed, f, w, 1) (RNG stream 1 of DESIGN.md §9), bits at and beyond K cleared; its codeword is
+ *     dnaldpc_encode(message); its channel values are exactly what dnaldpc_synth_{bsc,awgn,vote}_device produce for frame
+ *     f given that codeword (vote counts: read_err = param, mean_reads); it is decoded as dnaldpc_decode_batch_device
+ *     decodes that input kind with param and flags (vote counts with the table built from eps = param).
+ *   Raw hard decision ("without coding"): BSC the received bit, AWGN y < 0, vote counts k < 0.
+ *   Stopping. With T = target_frame_errors > 0 the result counts the shortest prefix of frames [0, n) that holds T frame
+ *     errors, or n = max_frames if that comes first; with T = 0 exactly max_frames frames. Frames decoded past n are
+ *     discarded, so every counter is a function of (code, spec) alone, whatever the piece size, wave_frames, number of
+ *     GPUs or timing.
+ *   Requirements. The systematic form is required: codes over its cap give DNALDPC_ERR_UNSUPPORTED (as dnaldpc_encode).
+ *     DNALDPC_ERR_ARG, before any device work, for a null handle or pointer, an unknown channel or flag, p not in (0,1),
+ *     sigma <= 0, mean_reads not in (0,32] (vote counts), max_iter < 0, max_frames < 1 or target_frame_errors < 0.
+ *   Devices. Runs on every device of the decoder like a batch call (each device encodes its own frames with an encoder
+ *     of its own); dnaldpc_get_stats reports every frame decoded, the discarded ones included. Blocking. */
+typedef struct dnaldpc_sim {
+    int32_t channel;   /* DNALDPC_IN_BSC_BITS (param = p), DNALDPC_IN_AWGN_F32 (param = sigma),
+                          DNALDPC_IN_VOTE_I8 (param = read error probability, also the decoder's eps; mean_reads) */
+    int32_t flags;     /* DNALDPC_FLAG_MINSUM, DNALDPC_FLAG_FIXED_ITERS; anything else -> DNALDPC_ERR_ARG */
+    double param, mean_reads;
+    uint64_t seed;
+    int32_t max_iter;
+    int64_t max_frames;           /* frames to simulate; the cap when target_frame_errors > 0 */
+    int64_t target_frame_errors;  /* 0 = exactly max_frames */
+} dnaldpc_sim;
+typedef struct dnaldpc_sim_result {
+    int64_t frames, iterations;                 /* frames counted; sum of their iteration counts          */
+    int64_t frame_errors, bit_errors;           /* decoded != sent, over all N bits                       */
+    int64_t msg_frame_errors, msg_bit_errors;   /* the same over the K info columns (the message)          */
+    int64_t detected, undetected;               /* syndrome != 0 / syndrome == 0 but decoded != sent       */
+    int64_t raw_frame_errors, raw_bit_errors;   /* channel hard decision != sent ("without coding")        */
+} dnaldpc_sim_result;
+int dnaldpc_simulate(dnaldpc_decoder *d, const dnaldpc_sim *s, dnaldpc_sim_result *r);
+
 /* ---- statistics of the last decode call on this handle ------------------------------------------ */
 typedef struct dnaldpc_stats {
     int64_t frames;
