@@ -18,6 +18,7 @@ IN_LR_F64, IN_LLR_F64, IN_BSC_BITS, IN_AWGN_F32, IN_AWGN_F64, IN_VOTE_I8 = range
 FLAG_HOST_EXP = 1
 FLAG_FIXED_ITERS = 2
 FLAG_MINSUM = 4
+FLAG_LAYERED = 8  # with FLAG_MINSUM: row-layered normalised min-sum (include/dnaldpc.h)
 
 EXPORTS = [
     "dnaldpc_last_error", "dnaldpc_version", "dnaldpc_code_read_pchk", "dnaldpc_code_from_csr",
@@ -28,6 +29,7 @@ EXPORTS = [
     "dnaldpc_selftest_math", "dnaldpc_redecode_sweep", "dnaldpc_get_trace", "dnaldpc_decode_window",
     "dnaldpc_redecode_sweep_ex", "dnaldpc_synth_awgn_device", "dnaldpc_synth_vote_device", "dnaldpc_code_systematic",
     "dnaldpc_encode_device", "dnaldpc_encode", "dnaldpc_extract_device", "dnaldpc_extract", "dnaldpc_simulate",
+    "dnaldpc_code_layers", "dnaldpc_set_minsum_scale",
 ]
 
 
@@ -125,6 +127,8 @@ def lib():
         for name in ("dnaldpc_encode", "dnaldpc_extract"):
             getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
         L.dnaldpc_simulate.argtypes = [C.c_void_p, C.POINTER(Sim), C.POINTER(SimResult)]
+        L.dnaldpc_code_layers.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_void_p]
+        L.dnaldpc_set_minsum_scale.argtypes = [C.c_void_p, C.c_double]
         _lib = L
     return _lib
 
@@ -178,6 +182,13 @@ class Code:
             _check(lib().dnaldpc_code_systematic(self._h, C.byref(K), info.ctypes.data, par.ctypes.data))
             self._sys = (info[:K.value].copy(), par[:self.N - K.value].copy())
         return self._sys
+
+    def layers(self):
+        """(n_layers, layer_of_row int32 [M]) of the layered decoder's first-fit row layers (include/dnaldpc.h)."""
+        n = C.c_int()
+        lay = np.zeros(self.M, np.int32)
+        _check(lib().dnaldpc_code_layers(self._h, C.byref(n), lay.ctypes.data))
+        return n.value, lay
 
 
 def _pack_bits(bits):
@@ -387,6 +398,10 @@ class Decoder:
         r = SimResult()
         _check(lib().dnaldpc_simulate(self._h, C.byref(spec), C.byref(r)))
         return {k: getattr(r, k) for k, _ in SimResult._fields_}
+
+    def set_minsum_scale(self, alpha):
+        """Normalisation alpha in (0, 1] of the layered min-sum decoder (FLAG_MINSUM | FLAG_LAYERED); default 1."""
+        _check(lib().dnaldpc_set_minsum_scale(self._h, float(alpha)))
 
     def stats(self):
         s = Stats()

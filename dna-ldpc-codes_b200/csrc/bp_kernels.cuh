@@ -99,7 +99,7 @@ __device__ __forceinline__ void row_compute(T (&d)[DC], int deg, T *base, const 
 //   decision (Decision_MSA_INF, dec.cpp:1659-1677): L = LLR + sum_m c2v_m; bit = !(L > 0)
 // Same slot layout and scheduler; `lratio` holds the channel LLR, `msg` holds v2c before / c2v after the check pass.
 // ------------------------------------------------------------------------------------------------
-enum Alg { ALG_BP = 0, ALG_MINSUM = 1 };
+enum Alg { ALG_BP = 0, ALG_MINSUM = 1, ALG_LAYERED = 2 /* setup / harvest only: layered_kernels.cuh */ };
 
 template <typename T, int DC, bool EXACT>
 __device__ __forceinline__ void row_compute_minsum(T (&d)[DC], int deg, T *base) {
@@ -1046,6 +1046,9 @@ syndrome_update_half_kernel(const uint32_t *__restrict__ decw, SchedArrays s, Sy
 //            counts} (DNA_main.cpp:1340-1345, channel.cpp:32-33,75-84, decoder.py:314), transposed through shared
 //            memory into the slot-interleaved lratio array, and the initial decision lratio < 1 (dec.cpp:626).
 // ------------------------------------------------------------------------------------------------
+// Channel LLRs of the layered decoder are clamped to +-2^64 (and NaN set to 0) where they become the posterior q.
+constexpr double kLayeredLlrMax = 18446744073709551616.0;
+
 enum InKind { IN_LR_F64 = 0, IN_LLR_F64 = 1, IN_BSC_BITS = 2, IN_AWGN_F32 = 3, IN_AWGN_F64 = 4, IN_VOTE_I8 = 5 };
 
 struct SetupArgs {
@@ -1154,7 +1157,7 @@ harvest_setup_kernel(SetupArgs a, HarvestArgs h, SchedArrays s, T *__restrict__ 
                     const int r = __ffs(m) - 1;
                     const int fr = __shfl_sync(0xffffffffu, my_new, r);
                     double v = 1.0;
-                    if (j < N) v = ALG == ALG_MINSUM ? load_llr<KIND>(a, fr, j) : load_lr<KIND>(a, fr, j);
+                    if (j < N) v = ALG != ALG_BP ? load_llr<KIND>(a, fr, j) : load_lr<KIND>(a, fr, j);
                     tile[r][lane] = v;
                 }
                 __syncwarp();
@@ -1164,9 +1167,10 @@ harvest_setup_kernel(SetupArgs a, HarvestArgs h, SchedArrays s, T *__restrict__ 
                 const int jj = j0 + r;
                 double dv = 1.0;
                 if (is_new) dv = KIND == IN_BSC_BITS ? a.table[(bsc_word >> r) & 1u] : tile[lane][r];
-                const T v = ALG == ALG_MINSUM ? (T)dv : clamp_lr((T)dv);
+                T v = ALG != ALG_BP ? (T)dv : clamp_lr((T)dv);
+                if (ALG == ALG_LAYERED) v = v != v ? T(0) : (v < -(T)kLayeredLlrMax ? -(T)kLayeredLlrMax : (v > (T)kLayeredLlrMax ? (T)kLayeredLlrMax : v));
                 // initial decision: BP lratio < 1 (dec.cpp:626); min-sum !(LLR > 0) (Init_MSA_INF, dec.cpp:1311-1312)
-                const uint32_t w = __ballot_sync(0xffffffffu, ALG == ALG_MINSUM ? !(v > T(0)) : (v < T(1)));
+                const uint32_t w = __ballot_sync(0xffffffffu, ALG != ALG_BP ? !(v > T(0)) : (v < T(1)));
                 if (lane == r) wmine = w;
                 if (jj < N && is_new) lratio[((size_t)g * N + jj) * kFG + lane] = v;
             }

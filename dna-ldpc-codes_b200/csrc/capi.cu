@@ -10,6 +10,7 @@
 
 #include "../../include/dnaldpc.h"
 #include "../host/code.h"
+#include "../host/layers.h"
 #include "../host/systematic.h"
 #include "encoder.h"
 #include "engine.h"
@@ -114,6 +115,14 @@ int dnaldpc_code_check_regular(const dnaldpc_code *c, int *dv, int *regular_dv, 
     return DNALDPC_OK;
 }
 
+int dnaldpc_code_layers(const dnaldpc_code *c, int *n_layers, int32_t *layer_of_row) {
+    if (!c || !n_layers) return set_err(DNALDPC_ERR_ARG, "null argument");
+    const Layers &l = code_layers(c->c);
+    *n_layers = l.n_layers;
+    if (layer_of_row) memcpy(layer_of_row, l.layer_of_row.data(), l.layer_of_row.size() * 4);
+    return DNALDPC_OK;
+}
+
 int dnaldpc_decoder_create(const dnaldpc_code *c, const dnaldpc_config *cfg, dnaldpc_decoder **out) {
     DeviceRestore restore_device;
     if (!c || !out) return set_err(DNALDPC_ERR_ARG, "null argument");
@@ -155,6 +164,20 @@ void dnaldpc_decoder_destroy(dnaldpc_decoder *d) {
     delete d;
 }
 
+int dnaldpc_set_minsum_scale(dnaldpc_decoder *d, double alpha) {
+    if (!d) return set_err(DNALDPC_ERR_ARG, "null decoder");
+    if (!(alpha > 0.0 && alpha <= 1.0)) return set_err(DNALDPC_ERR_ARG, "min-sum scale must be in (0, 1]");
+    for (auto &e : d->eng) e->minsum_scale = alpha;
+    return DNALDPC_OK;
+}
+
+// DNALDPC_FLAG_LAYERED exists for min-sum only (a layered sum-product is not implemented).
+static int check_layered(int flags) {
+    if ((flags & DNALDPC_FLAG_LAYERED) && !(flags & DNALDPC_FLAG_MINSUM))
+        return set_err(DNALDPC_ERR_UNSUPPORTED, "DNALDPC_FLAG_LAYERED needs DNALDPC_FLAG_MINSUM (no layered sum-product)");
+    return DNALDPC_OK;
+}
+
 static int check_input(const dnaldpc_input *in, int N) {
     if (!in) return set_err(DNALDPC_ERR_ARG, "null input descriptor");
     if (packed_stride(in->kind, N) == 0) return set_err(DNALDPC_ERR_ARG, "unknown input kind");
@@ -164,7 +187,7 @@ static int check_input(const dnaldpc_input *in, int N) {
         return set_err(DNALDPC_ERR_ARG, "AWGN sigma must be positive");
     if (in->kind == DNALDPC_IN_VOTE_I8 && !in->table && !(in->param > 0.0 && in->param < 1.0))
         return set_err(DNALDPC_ERR_ARG, "vote-count eps must be in (0,1)");
-    return DNALDPC_OK;
+    return check_layered(in->flags);
 }
 
 int dnaldpc_decode_batch(dnaldpc_decoder *d, const dnaldpc_input *in, int64_t F, int max_iter, const dnaldpc_output *out) {
@@ -468,7 +491,9 @@ int dnaldpc_simulate(dnaldpc_decoder *d, const dnaldpc_sim *s, dnaldpc_sim_resul
     if (!d || !s || !r) return set_err(DNALDPC_ERR_ARG, "null argument");
     if (s->channel != DNALDPC_IN_BSC_BITS && s->channel != DNALDPC_IN_AWGN_F32 && s->channel != DNALDPC_IN_VOTE_I8)
         return set_err(DNALDPC_ERR_ARG, "unknown simulation channel (BSC_BITS, AWGN_F32 or VOTE_I8)");
-    if (s->flags & ~(DNALDPC_FLAG_MINSUM | DNALDPC_FLAG_FIXED_ITERS)) return set_err(DNALDPC_ERR_ARG, "unknown simulation flag");
+    if (s->flags & ~(DNALDPC_FLAG_MINSUM | DNALDPC_FLAG_FIXED_ITERS | DNALDPC_FLAG_LAYERED))
+        return set_err(DNALDPC_ERR_ARG, "unknown simulation flag");
+    if (int rc = check_layered(s->flags)) return rc;
     if ((s->channel == DNALDPC_IN_BSC_BITS || s->channel == DNALDPC_IN_VOTE_I8) && !(s->param > 0.0 && s->param < 1.0))
         return set_err(DNALDPC_ERR_ARG, "error probability must be in (0,1)");
     if (s->channel == DNALDPC_IN_AWGN_F32 && !(s->param > 0.0)) return set_err(DNALDPC_ERR_ARG, "AWGN sigma must be positive");

@@ -8,7 +8,9 @@
 #include <cstring>
 #include <thread>
 
+#include "../host/layers.h"
 #include "bp_kernels.cuh"
+#include "layered_kernels.cuh"
 #include "sw_kernels.cuh"
 
 namespace dnaldpc {
@@ -62,6 +64,12 @@ Engine::Engine(const Code &code, int device, int precision, int wave_frames)
     up(&d_col_idx_, code.col_idx);
     up(&d_col_ptr_, code.col_ptr);
     up(&d_col_edge_, code.col_edge);
+    const Layers &lay = code_layers(code);
+    up(&d_layer_rows_, lay.rows);
+    layer_ptr_ = lay.ptr;
+    for (int j = 0; j < N_; j++) empty_cols_ = empty_cols_ || code.col_ptr[(size_t)j + 1] == code.col_ptr[(size_t)j];
+    const int dc = layer_dc(max_row_deg_);
+    layer_w_ = esz_ == 4 ? layer_state_w<float>(dc) : layer_state_w<double>(dc);
     chk(cudaMalloc((void **)&d_table_, 256 * sizeof(double)), "cudaMalloc(table)");
     chk(cudaMalloc((void **)&d_next_, 3 * sizeof(unsigned long long)), "cudaMalloc(next)");
     chk(cudaMalloc((void **)&d_counters_, ((size_t)kRing * kCounterWords + 1) * sizeof(unsigned)), "cudaMalloc(counters)");  // + the check pass's job counter
@@ -78,7 +86,7 @@ Engine::Engine(const Code &code, int device, int precision, int wave_frames)
 Engine::~Engine() {
     cudaSetDevice(device_);
     cudaDeviceSynchronize();
-    void *ptrs[] = {d_row_ptr_, d_col_idx_, d_col_ptr_, d_col_edge_, d_msg_, d_lratio_, d_post_, d_decw_, d_masks_, d_arrive_,
+    void *ptrs[] = {d_row_ptr_, d_col_idx_, d_col_ptr_, d_col_edge_, d_layer_rows_, d_msg_, d_lratio_, d_post_, d_decw_, d_masks_, d_arrive_,
                     d_slot_, d_mv_, d_sw_lr_, d_edge_row_, d_next_, d_iters_, d_ok_, d_table_, d_counters_, s_in_, s_bits_, s_dblk_, s_post_, s_pchk_,
                     s_iters_, s_ok_, d_rows_, d_synth_thr_, d_list_[0], d_list_[1], d_col_row_, d_sw_sched_, s_in2_, d_sw_avail_, d_sw_lists_, d_sw_thin_, d_sw_hist_};
     for (void *p : ptrs) if (p) cudaFree(p);
@@ -101,7 +109,9 @@ int Engine::ensure_slots(int G, bool want_post) {
         for (void *p : ptrs) if (p) cudaFree(p);
         d_msg_ = d_lratio_ = d_post_ = nullptr; d_decw_ = d_masks_ = nullptr; d_arrive_ = nullptr; d_slot_ = d_mv_ = nullptr;
         cap_groups_ = 0;
-        CK(cudaMalloc(&d_msg_, std::max<size_t>((size_t)G * E_ * kFG * esz_, 16)));
+        // per slot: E flooding messages, or M * layer_w_ elements of layered check state
+        const size_t msg_elems = std::max<size_t>((size_t)E_, (size_t)M_ * layer_w_);
+        CK(cudaMalloc(&d_msg_, std::max<size_t>((size_t)G * msg_elems * kFG * esz_, 16)));
         CK(cudaMalloc(&d_lratio_, (size_t)G * N_ * kFG * esz_));
         CK(cudaMalloc((void **)&d_decw_, (size_t)G * N_ * sizeof(uint32_t)));
         CK(cudaMalloc((void **)&d_masks_, (size_t)G * 6 * sizeof(uint32_t)));
@@ -246,6 +256,28 @@ template <typename T> int Engine::launch_col(int g0, int G, bool want_post, cuda
     return DNALDPC_OK;
 }
 
+// One layered min-sum iteration of groups [0, G): one launch per layer, in ascending layer order.
+template <typename T> int Engine::launch_layers(int G, cudaStream_t st) {
+    SchedArrays s;
+    fill_sched(s);
+    const T alpha = (T)minsum_scale;
+    const int dc = layer_dc(max_row_deg_);
+    for (size_t l = 0; l + 1 < layer_ptr_.size(); l++) {
+        const int r0 = layer_ptr_[l], nrows = layer_ptr_[l + 1] - r0;
+        if (nrows == 0) continue;
+        const unsigned grid = (unsigned)(((long long)G * nrows + kRowWarps - 1) / kRowWarps);
+#define LAY(DC, KEEP) layer_pass_kernel<T, DC, KEEP><<<grid, kRowWarps * 32, 0, st>>>((T *)d_msg_, (T *)d_lratio_, d_decw_, s.actw, s.freshw, d_row_ptr_, d_col_idx_, d_layer_rows_ + r0, nrows, M_, N_, 0, G, alpha)
+        if (dc == 8) LAY(8, true);
+        else if (dc == 32) LAY(32, true);
+        else if (dc == 72) LAY(72, true);
+        else LAY(128, sizeof(T) == 4);
+#undef LAY
+        stats.kernel_launches++;
+    }
+    CK(cudaGetLastError());
+    return DNALDPC_OK;
+}
+
 // check() + loop control for the slots under consideration (syndrome_update_*_kernel)
 int Engine::launch_syndrome(const dnaldpc_output &out, int G, int max_iter, int consider_new, int fixed, unsigned *counter,
                             unsigned *finished, unsigned *rearm, int clear_fresh, cudaStream_t st) {
@@ -302,10 +334,11 @@ int Engine::launch_harvest_setup(const dnaldpc_input &in, const dnaldpc_output &
     const int tiles_per_cta = kHsWarps * tpw;
     dim3 grid((unsigned)(((N_ + 31) / 32 + tiles_per_cta - 1) / tiles_per_cta), (unsigned)G);
     T *lr = (T *)d_lratio_;
-    const T *post = (const T *)d_post_;
+    const T *post = layered_ ? lr : (const T *)d_post_;  // the layered decoder's posterior is q, kept in lratio
 #define HS(K)                                                                                                   \
     do {                                                                                                        \
-        if (minsum_) harvest_setup_kernel<T, K, ALG_MINSUM><<<grid, kHsWarps * 32, 0, st>>>(a, h, s, lr, post, d_decw_, N_, g0, tpw); \
+        if (layered_) harvest_setup_kernel<T, K, ALG_LAYERED><<<grid, kHsWarps * 32, 0, st>>>(a, h, s, lr, post, d_decw_, N_, g0, tpw); \
+        else if (minsum_) harvest_setup_kernel<T, K, ALG_MINSUM><<<grid, kHsWarps * 32, 0, st>>>(a, h, s, lr, post, d_decw_, N_, g0, tpw); \
         else harvest_setup_kernel<T, K, ALG_BP><<<grid, kHsWarps * 32, 0, st>>>(a, h, s, lr, post, d_decw_, N_, g0, tpw);         \
     } while (0)
     switch (in.kind) {
@@ -383,7 +416,9 @@ int Engine::run(const Session &ss, FrameSource &src, cudaStream_t st) {
     if (Fmax > 0x7fffffffLL) return fail("more than 2^31-1 frames in one call", DNALDPC_ERR_ARG);
     const int G = (int)std::min<int64_t>((Fmax + 31) / 32, wave_frames_ / 32);
     const long long S = (long long)G * kFG;
-    const bool want_post = ss.out.posterior != nullptr;
+    minsum_ = (in.flags & DNALDPC_FLAG_MINSUM) != 0;
+    layered_ = minsum_ && (in.flags & DNALDPC_FLAG_LAYERED) != 0;
+    const bool want_post = ss.out.posterior != nullptr && !layered_;  // flooding: the bit pass writes d_post_
     int rc = ensure_slots(G, want_post);
     if (rc) return rc;
     rc = ensure_rows(Fmax);
@@ -395,7 +430,6 @@ int Engine::run(const Session &ss, FrameSource &src, cudaStream_t st) {
         if (!out.iters) out.iters = d_iters_;
         if (!out.is_codeword) out.is_codeword = d_ok_;
     }
-    minsum_ = (in.flags & DNALDPC_FLAG_MINSUM) != 0;
     if (in.kind == DNALDPC_IN_BSC_BITS || in.kind == DNALDPC_IN_VOTE_I8) {
         double tab[256];
         int cnt = 256;
@@ -493,14 +527,18 @@ int Engine::run(const Session &ss, FrameSource &src, cudaStream_t st) {
                 src.wait_for_frames();
                 last_admitted = 1;  // look for frames in the next tick
             }
-            if (!no_compact && !profiling && final && admitted_total == published() && packed_cap >= 2 * kFG &&
+            // (layered decodes of a code with empty columns are not compacted: compact_move_kernel does not move decision
+            // words, and no layer pass rewrites those columns' words in the destination slot)
+            if (!no_compact && !profiling && !(layered_ && empty_cols_) && final && admitted_total == published() && packed_cap >= 2 * kFG &&
                 (long long)last_inuse * 100 <= packed_cap * compact_pct) {
                 // `last_inuse` is kLag ticks old and can only have shrunk since: it bounds the moves and the packed size
                 int32_t *mv_src = d_mv_, *mv_dst = d_mv_ + (size_t)cap_groups_ * kFG, *mv_cnt = d_mv_ + (size_t)cap_groups_ * kFG * 2;
                 compact_plan_kernel<<<1, 32, 0, st>>>(s, G, mv_src, mv_dst, mv_cnt);
-                dim3 mgrid((unsigned)((E_ + N_ + kMoveThreads * kMoveUnroll - 1) / (kMoveThreads * kMoveUnroll)),
+                const int msg_elems = layered_ ? M_ * layer_w_ : E_;
+                dim3 mgrid((unsigned)((msg_elems + N_ + kMoveThreads * kMoveUnroll - 1) / (kMoveThreads * kMoveUnroll)),
                            (unsigned)std::min<unsigned>(std::max(last_inuse, 1u), 2048u));
-                compact_move_kernel<T><<<mgrid, kMoveThreads, 0, st>>>((T *)d_msg_, (T *)d_lratio_, mv_src, mv_dst, mv_cnt, N_, E_);
+                // per slot: the E messages, or the M * layer_w_ elements of layered check state, and lratio (q)
+                compact_move_kernel<T><<<mgrid, kMoveThreads, 0, st>>>((T *)d_msg_, (T *)d_lratio_, mv_src, mv_dst, mv_cnt, N_, msg_elems);
                 stats.kernel_launches += 2;
                 stats.compactions++;
                 CK(cudaGetLastError());
@@ -512,11 +550,11 @@ int Engine::run(const Session &ss, FrameSource &src, cudaStream_t st) {
         const bool trace = trace_ticks_ > 0 && tick >= 8 && tick < 8 + kTrace && tick < 8 + trace_ticks_;  // in-pipeline timing, no sync
         if (trace) CK(cudaEventRecord(trace_ev_[3 * (tick - 8)], st));
         if (profiling) CK(cudaEventRecord(prof_ev_[0], st));
-        rc = launch_row<T>(0, G_rc, st);
+        rc = layered_ ? launch_layers<T>(G_rc, st) : launch_row<T>(0, G_rc, st);  // layered: the layer passes count as the check pass
         if (rc) return rc;
         if (profiling) CK(cudaEventRecord(prof_ev_[1], st));
         if (trace) CK(cudaEventRecord(trace_ev_[3 * (tick - 8) + 1], st));
-        rc = launch_col<T>(0, G_rc, want_post, st);
+        if (!layered_) rc = launch_col<T>(0, G_rc, want_post, st);
         if (rc) return rc;
         if (trace) { CK(cudaEventRecord(trace_ev_[3 * (tick - 8) + 2], st)); traced_ = (int)(tick - 8) + 1; }
         if (profiling) {

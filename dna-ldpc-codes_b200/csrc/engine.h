@@ -77,6 +77,7 @@ class Engine {
 
     dnaldpc_stats stats{};
     bool profiling = false;
+    double minsum_scale = 1.0;  // alpha of the layered min-sum decoder (dnaldpc_set_minsum_scale)
     int trace_ticks_ = 0;  // > 0: record in-pipeline events for that many ticks of the next batch (no synchronisation)
     int trace_result(double *row_ms, double *col_ms, double *sched_ms);
 
@@ -89,6 +90,7 @@ class Engine {
     int ensure_rows(int64_t frames);
     template <typename T> int launch_row(int g0, int G, cudaStream_t st);
     template <typename T> int launch_col(int g0, int G, bool want_post, cudaStream_t st);
+    template <typename T> int launch_layers(int G, cudaStream_t st);
     template <typename T> int launch_harvest_setup(const dnaldpc_input &in, const dnaldpc_output &out, int g0, int G, cudaStream_t st);
     int launch_syndrome(const dnaldpc_output &out, int G, int max_iter, int consider_new, int fixed, unsigned *counter,
                         unsigned *finished, unsigned *rearm, int clear_fresh, cudaStream_t st);
@@ -105,9 +107,15 @@ class Engine {
     bool smem_attr_set_[2] = {false, false}, syn_attr_set_ = false, tmem_attr_set_ = false, syn_half_attr_set_ = false;
     bool steady_ = false;  // last polled tick: all slots busy, no frame admitted
     bool minsum_ = false;  // current batch runs the LLR-domain min-sum rules instead of sum-product
+    bool layered_ = false; // current batch runs layered normalised min-sum (layered_kernels.cuh)
     size_t esz_ = 8;
     // H edge tables (device)
     int32_t *d_row_ptr_ = nullptr, *d_col_idx_ = nullptr, *d_col_ptr_ = nullptr, *d_col_edge_ = nullptr;
+    // row layers (host/layers.h): rows grouped by layer (device) and the layer offsets (host)
+    int32_t *d_layer_rows_ = nullptr;
+    std::vector<int32_t> layer_ptr_;
+    int layer_w_ = 0;  // T-sized elements of one check's layered state (LayerState<T, DC>::W of this code)
+    bool empty_cols_ = false;  // some column has no entry: no layer pass rewrites its decision word
     // slot state (device)
     int cap_groups_ = 0;
     void *d_msg_ = nullptr, *d_lratio_ = nullptr, *d_post_ = nullptr;

@@ -3,6 +3,7 @@
 #include <algorithm>
 #include <cstdio>
 
+#include "layers.h"
 #include "systematic.h"
 
 namespace dnaldpc {
@@ -10,6 +11,7 @@ namespace dnaldpc {
 std::string build_code(int M, int N, std::vector<int64_t> &pairs, Code &c) {
     if (M <= 0 || N <= 0) return "matrix dimensions must be positive";
     c.sys = std::make_shared<SystematicCache>();
+    c.layers = std::make_shared<LayersCache>();
     std::sort(pairs.begin(), pairs.end());
     pairs.erase(std::unique(pairs.begin(), pairs.end()), pairs.end());  // insert() merges duplicates (mod2sparse.cpp:521-524)
     c.M = M; c.N = N; c.E = (int)pairs.size();

@@ -11,6 +11,7 @@
 namespace dnaldpc {
 
 struct SystematicCache;
+struct LayersCache;
 
 struct Code {
     int M = 0, N = 0, E = 0;
@@ -21,6 +22,7 @@ struct Code {
     int max_row_deg = 0, max_col_deg = 0;
     bool regular_rows = true, regular_cols = true;
     std::shared_ptr<SystematicCache> sys;  // systematic form (host/systematic.h), computed on first use
+    std::shared_ptr<LayersCache> layers;   // row layers of the layered decoder (host/layers.h), computed on first use
 };
 
 // Build from (row, col) pairs in any order with duplicates; returns error text or "".

@@ -27,17 +27,20 @@
 //                     same stdout, same exit code); otherwise it runs locally. The unmodified pipeline
 //                     (ex_decoder/def_func.py:47-51, one os.system("ldpc ...") per codeword) then pays milliseconds
 //                     per call instead of a CUDA context creation.
+//   --layered         with decoder types 20-22: row-layered normalised min-sum (DNALDPC_FLAG_LAYERED) instead of the
+//                     flooding min-sum; --scale A sets its normalisation alpha in (0, 1] (default 1)
 //
 // Simulation (the reference's frame_num / target_frame_err mode: random codewords through a synthetic channel):
 //   ldpc --simulate <pchk_base> <channel_type> <p1[,p2,...]> <seed> <max_iter> <frame_num> [<target_frame_err> if frame_num==0]
-//        [--max-frames N] [--reads R] [--decoder 0|20] [--device N] [--gpus N] [--fp32] [--timing]
+//        [--max-frames N] [--reads R] [--decoder 0|20] [--layered [--scale A]] [--device N] [--gpus N] [--fp32] [--timing]
 // runs dnaldpc_simulate once per parameter: frames carry random messages (RNG stream 1 of DESIGN.md §9) encoded with
 // the systematic form, go through the channel and are decoded and counted on the GPU. Channel types: 0 = AWGN, the
 // parameters are Eb/N0 in dB and sigma = getStd_dev(Eb/N0, K/N) with K = N - rank(H), the true rate of the code;
 // 1 = BSC with crossover probability p; 3 = vote counts of aligned reads, p = read error probability (also the
 // decoder's eps), --reads R mean reads per bit (required, in (0, 32]). 2 (BEC) and anything else are rejected.
 // frame_num > 0 simulates exactly that many frames; frame_num 0 runs until <target_frame_err> frame errors, capped by
-// --max-frames (default 10^9). --decoder 20 decodes with floating min-sum. Per parameter a Print_One_Result block
+// --max-frames (default 10^9). --decoder 20 decodes with floating min-sum, --decoder 20 --layered with layered
+// normalised min-sum (--scale A: alpha). Per parameter a Print_One_Result block
 // (DNA_main.cpp:1170-1182) plus msg_bit_err, undetected (zero syndrome, wrong codeword) and avg_iter lines; --timing
 // adds one JSON line per parameter on stderr with every counter and the wall time. Argument and file errors are
 // reported before any CUDA call.
@@ -89,6 +92,8 @@ struct Args {
     std::string msg_base;  // --encode: <pchk_base> <msg_base> <codeword_base> (cw_base, pchk_base as for decoding)
     std::vector<std::string> sim_pos;  // --simulate: the positional arguments after the flag
     std::string max_frames, reads, decoder;  // --simulate options, checked by run_simulate
+    bool layered = false;                    // --layered: DNALDPC_FLAG_LAYERED (min-sum decoders only)
+    std::string scale;                       // --scale A: normalisation of the layered decoder, checked by check_layered
 };
 
 // Where a run writes: a local run uses the process's own streams, a run on behalf of a client memory streams.
@@ -114,6 +119,8 @@ bool parse(const std::vector<std::string> &argv, Args &a, Io &io) {
         else if (s == "--max-frames" && i + 1 < argv.size()) a.max_frames = argv[++i];
         else if (s == "--reads" && i + 1 < argv.size()) a.reads = argv[++i];
         else if (s == "--decoder" && i + 1 < argv.size()) a.decoder = argv[++i];
+        else if (s == "--layered") a.layered = true;
+        else if (s == "--scale" && i + 1 < argv.size()) a.scale = argv[++i];
         else pos.push_back(s);
     }
     if (a.serve || a.shutdown) return true;
@@ -157,6 +164,19 @@ bool parse(const std::vector<std::string> &argv, Args &a, Io &io) {
     return true;
 }
 
+bool parse_num(const std::string &s, double &v);
+
+// --layered / --scale: the layered decoder exists for min-sum only; alpha in (0, 1]. Returns the error text or "".
+std::string check_layered(const Args &a, bool minsum, double &alpha) {
+    alpha = 1.0;
+    if (a.layered && !minsum) return "--layered needs a min-sum decoder (decoder type 20-22, --simulate --decoder 20)";
+    if (!a.scale.empty()) {
+        if (!a.layered) return "--scale needs --layered";
+        if (!parse_num(a.scale, alpha) || !(alpha > 0.0 && alpha <= 1.0)) return "--scale must be in (0, 1]";
+    }
+    return "";
+}
+
 // Decoders kept by the resident worker: one per (parity-check file, its size and modification time, precision, GPUs).
 struct Cache {
     struct Entry { dnaldpc_code *code; dnaldpc_decoder *dec; };
@@ -180,6 +200,11 @@ int run(Args a, Io &io, Cache *cache) {
     if (a.decoder_type != 0 && !minsum && !window) {
         fprintf(io.err, "ldpc: decoder type %d is not supported by this build (0 = belief propagation, 20-22 = floating min-sum, 60 = sliding window)\n", a.decoder_type);
         return 1;
+    }
+    double alpha = 1.0;
+    {
+        const std::string why = check_layered(a, minsum, alpha);
+        if (!why.empty()) { fprintf(io.err, "ldpc: %s\n", why.c_str()); return 1; }
     }
     if (a.punctuation || a.shortening || a.targeting) {
         fprintf(io.err, "ldpc: punctuation / shortening / targeting are not supported by this build (pass 0 0 0)\n");
@@ -328,7 +353,9 @@ int run(Args a, Io &io, Cache *cache) {
     dnaldpc_input in{};
     in.kind = minsum ? DNALDPC_IN_LLR_F64 : DNALDPC_IN_LR_F64;   // min-sum works on the LLRs themselves
     in.flags = minsum ? DNALDPC_FLAG_MINSUM : 0;
+    if (a.layered) in.flags |= DNALDPC_FLAG_LAYERED;
     in.data = minsum ? llr.data() : lr.data();
+    CHECK(dnaldpc_set_minsum_scale(dec, alpha));  // every run: a resident decoder keeps the previous run's value
     dnaldpc_output out{};
     out.dblk = dblk.data();
     out.iters = iters.data();
@@ -511,7 +538,7 @@ int run_encode(Args a, Io &io, bool resident) {
 // ldpc --simulate: one dnaldpc_simulate call per channel parameter.
 const char kSimUsage[] =
     "usage: ldpc --simulate <pchk_base> <channel_type> <p1[,p2,...]> <seed> <max_iter> <frame_num> [<target_frame_err> if frame_num==0]\n"
-    "                       [--max-frames N] [--reads R] [--decoder 0|20] [--device N] [--gpus N] [--fp32] [--timing]\n"
+    "                       [--max-frames N] [--reads R] [--decoder 0|20] [--layered [--scale A]] [--device N] [--gpus N] [--fp32] [--timing]\n"
     "  channel_type 0: AWGN, parameters Eb/N0 in dB, sigma from the true rate K/N (K = N - rank(H))\n"
     "               1: BSC, parameters crossover probabilities p\n"
     "               3: vote counts, parameters read error probabilities, --reads = mean reads per bit (required)\n";
@@ -570,6 +597,12 @@ int run_simulate(Args a, Io &io, bool resident) {
         if (a.decoder != "20") return usage("--decoder must be 0 (belief propagation) or 20 (floating min-sum)");
         flags = DNALDPC_FLAG_MINSUM;
     }
+    double alpha = 1.0;
+    {
+        const std::string why = check_layered(a, flags != 0, alpha);
+        if (!why.empty()) return usage(why.c_str());
+    }
+    if (a.layered) flags |= DNALDPC_FLAG_LAYERED;
     if (a.device < 0) return usage("--device must be >= 0");
     if (a.gpus < 1 || a.gpus > 16) return usage("--gpus must be between 1 and 16");
 
@@ -595,7 +628,10 @@ int run_simulate(Args a, Io &io, bool resident) {
     cfg.n_devices = a.gpus;
     for (int k = 0; k < a.gpus; k++) cfg.devices[k] = a.device + k;
     cfg.precision = a.fp32 ? DNALDPC_PREC_F32 : DNALDPC_PREC_F64;
-    if (dnaldpc_decoder_create(code, &cfg, &dec) != DNALDPC_OK) { fprintf(io.err, "%s\n", dnaldpc_last_error()); return 1; }
+    if (dnaldpc_decoder_create(code, &cfg, &dec) != DNALDPC_OK || dnaldpc_set_minsum_scale(dec, alpha) != DNALDPC_OK) {
+        fprintf(io.err, "%s\n", dnaldpc_last_error());
+        return 1;
+    }
     fprintf(io.out, "\ng_CODE_N : %d\ng_CODE_K : %d\ng_CODE_M : %d\n\n", N, K, M);
     for (size_t i = 0; i < params.size(); i++) {
         dnaldpc_sim sp{};

@@ -56,6 +56,11 @@ int dnaldpc_code_export(const dnaldpc_code *c, int32_t *row_ptr, int32_t *col_id
 /* CheckRegular (dec.cpp:138-189): max degrees D_v, D_c and the two regularity flags. */
 int dnaldpc_code_check_regular(const dnaldpc_code *c, int *dv, int *regular_dv, int *dc, int *regular_dc);
 
+/* Row layers of the layered decoder: the rows in ascending order, each in the lowest-numbered layer that holds no row
+ * sharing a column with it (first fit); a row without entries goes to layer 0. The checks of one layer touch disjoint
+ * bits. *n_layers receives the number of layers, layer_of_row[M] (may be NULL) each row's layer. Host only, no GPU needed. */
+int dnaldpc_code_layers(const dnaldpc_code *c, int *n_layers, int32_t *layer_of_row);
+
 /* ---- decoder --------------------------------------------------------------------------------- */
 
 #define DNALDPC_PREC_F64 0 /* bit-exact mode */
@@ -71,6 +76,9 @@ typedef struct dnaldpc_config {
 
 int dnaldpc_decoder_create(const dnaldpc_code *c, const dnaldpc_config *cfg, dnaldpc_decoder **out);
 void dnaldpc_decoder_destroy(dnaldpc_decoder *d);
+/* Normalisation alpha of the layered min-sum decoder (DNALDPC_FLAG_LAYERED), in (0, 1]; default 1 (plain min-sum).
+ * Used by layered decodes only. DNALDPC_ERR_ARG outside (0, 1]. */
+int dnaldpc_set_minsum_scale(dnaldpc_decoder *d, double alpha);
 
 /* Input kinds = the reference's "channel options" (likelihood setup; SURVEY.md §8a):                      */
 #define DNALDPC_IN_LR_F64 0   /* double [F][N]  lratio = p0/p1                  (g_received_LR, DNA_main.cpp:1344)          */
@@ -94,6 +102,22 @@ void dnaldpc_decoder_destroy(dnaldpc_decoder *d);
  * (Decision_MSA_INF, dec.cpp:1659-1677); a user table for VOTE_I8 must hold LLRs. LR_F64 inputs are converted with the
  * device log() and AWGN / LLR / BSC / vote-count inputs are exact. */
 #define DNALDPC_FLAG_MINSUM 4
+/* Row-layered schedule; only together with DNALDPC_FLAG_MINSUM: layered normalised min-sum (without MINSUM
+ * DNALDPC_ERR_UNSUPPORTED, reserved for a layered sum-product). Accepted by dnaldpc_decode_batch[_device],
+ * dnaldpc_redecode_sweep_ex and dnaldpc_simulate. Contract (T = the decoder's precision, fp64 or fp32):
+ *   Layers: dnaldpc_code_layers. One iteration runs the layers in ascending index.
+ *   lambda_j = the channel LLR of DNALDPC_FLAG_MINSUM for the input kind, rounded to T, NaN -> 0, clamped to +-2^64.
+ *   Init: q_j = lambda_j, c2v_e = 0, d_j = !(lambda_j > 0). Loop control as BP (c = weight(H*d); stop when n == max_iter
+ *   or c == 0, with FIXED_ITERS only at n == max_iter; else one iteration, n++).
+ *   Iteration: for each layer, for each check i of it and each edge e of i:
+ *     v_e = q_col(e) - c2v_e;  mu_e = min over e' != e of |v_e'| (0 if i has no other edge);
+ *     sigma_e = product over e' != e of (v_e' < 0 ? -1 : +1);  m = alpha * mu_e (one rounding in T, alpha = (T)scale);
+ *     c2v_e = sigma_e < 0 ? -m : m;  q_col(e) = clamp(v_e + c2v_e, +-2^64).   After the last layer d_j = !(q_j > 0).
+ *   Outputs: bits / dblk = d, iters = n, is_codeword = (c == 0), pchk = H*d, posterior = q (an LLR, widened to double).
+ *   Every step is one IEEE operation in T, so results do not depend on the thread mapping.
+ * The flooding DNALDPC_FLAG_MINSUM decoder ignores the scale. dnaldpc_decode_window takes no flags: the sliding-window
+ * decoder stays sum-product. */
+#define DNALDPC_FLAG_LAYERED 8
 
 typedef struct dnaldpc_input {
     int32_t kind;        /* DNALDPC_IN_* */
@@ -237,7 +261,8 @@ int dnaldpc_extract(dnaldpc_decoder *d, const uint32_t *cw, int64_t F, uint32_t 
 typedef struct dnaldpc_sim {
     int32_t channel;   /* DNALDPC_IN_BSC_BITS (param = p), DNALDPC_IN_AWGN_F32 (param = sigma),
                           DNALDPC_IN_VOTE_I8 (param = read error probability, also the decoder's eps; mean_reads) */
-    int32_t flags;     /* DNALDPC_FLAG_MINSUM, DNALDPC_FLAG_FIXED_ITERS; anything else -> DNALDPC_ERR_ARG */
+    int32_t flags;     /* DNALDPC_FLAG_MINSUM, DNALDPC_FLAG_FIXED_ITERS, DNALDPC_FLAG_LAYERED (with MINSUM);
+                          anything else -> DNALDPC_ERR_ARG */
     double param, mean_reads;
     uint64_t seed;
     int32_t max_iter;
